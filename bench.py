@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - DEER hot-path benchmark (BASELINE.json metric: train-step and inference samples/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One step = one pass of the hot path over one synthetic batch of the BASELINE shapes
@@ -13,7 +13,11 @@ One step = one pass of the hot path over one synthetic batch of the BASELINE sha
     D2H loss read inside the timed region;
   * `roofline`: the dominant kernel timed alone with CUDA events;
   * `cpu_baseline`: the stock-torch.nn CPU port of the reference path (oracle/torch_baseline.py) on a bounded sample.
-Prints ONE JSON line on rank 0.
+Prints ONE JSON line on rank 0.  The training, e2e, strong-scaling and inference loops each time exactly K steps.
+
+--dump-outputs DIR (rank 0) writes what the last timed training step computed, as float32 DIR/<name>.npy.  Inputs,
+weights and dropout masks are seeded, so two builds run with the same arguments can be compared file for file, within
+the run-to-run spread given in dump_outputs.
 """
 from __future__ import annotations
 
@@ -29,6 +33,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the checkout it runs from untouched (it may be read-only)
 
 TRAIN_B, INFER_B = 256, 1024
 TA, TV, TT = 300, 50, 64
@@ -173,7 +178,13 @@ def main():
                          "headline then reports scaling=strong.  Default 0: weak scaling, B=256 per GPU")
     ap.add_argument("--no-strong", action="store_true", help="skip the extra strong-scaling block (global batch 2048)")
     ap.add_argument("--no-loss-check", action="store_true", help="skip the step-0 loss check against the CPU port")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the GPU path; the reference arm has no such dump")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -308,6 +319,8 @@ def main():
 
     ms_per_step, launches_per_step, final_loss, clocks, NB = measure_train(B, K, W)
     value = B * world / (ms_per_step / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, args.dump_outputs, {"train_losses": trainer.last_losses, "train_params": trainer.flat.params})
     if args.train_only:
         if rank == 0:
             print(json.dumps({"metric": "deer_train_step_samples_per_s", "value": value, "ms_per_step": ms_per_step,
@@ -365,10 +378,9 @@ def main():
             strong_block = {"global_batch": STRONG_GLOBAL, "batch_per_gpu": Bs, "value": value,
                             "ms_per_step": ms_per_step, "unit": "samples/s", "note": "same run as the headline"}
         else:
-            sk = max(5, K // 4)
-            sms, _, _, _, _ = measure_train(Bs, sk, 3)
+            sms, _, _, _, _ = measure_train(Bs, K, 3)
             strong_block = {"global_batch": STRONG_GLOBAL, "batch_per_gpu": Bs, "value": STRONG_GLOBAL / (sms / 1e3),
-                            "ms_per_step": sms, "unit": "samples/s", "steps": sk}
+                            "ms_per_step": sms, "unit": "samples/s", "steps": K}
         trainer._graphs.clear()
         torch.cuda.empty_cache()
 
@@ -396,8 +408,7 @@ def main():
         else:
             infer_eager(ibatches[i % 2])
 
-    KI = max(3, K // 2)
-    infer_ms = timed(infer_fn, KI) / KI
+    infer_ms = timed(infer_fn, K) / K
     infer_value = INFER_B * world / (infer_ms / 1e3)
     del ibatches
     # inference end to end: pinned host batch (357 MB at B=1024) -> H2D -> forward -> D2H of the NIG parameters
@@ -429,7 +440,7 @@ def main():
     for i in range(3):
         infer_e2e(i)
     torch.cuda.synchronize()
-    infer_e2e_ms = timed(infer_e2e, KI) / KI
+    infer_e2e_ms = timed(infer_e2e, K) / K
     torch.cuda.synchronize()
     assert bool(torch.isfinite(nig_host[0]).all())
     infer_h2d = istager.bytes_per_batch
@@ -558,6 +569,29 @@ def check_loss_against_port(torch, model, dev, gen, Bc=16):
     rel = abs(got - ref) / max(abs(ref), 1e-12)
     assert rel <= 1e-3, f"bench loss check failed: GPU {got} vs CPU port {ref} (rel {rel:.2e})"
     return {"gpu": got, "cpu_port": ref, "rel_err": rel, "batch": Bc}
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(torch, path, arrays):
+    """Write {name: tensor} as float32 path/<name>.npy.
+
+    The benchmark dumps what the last timed training step hands its caller: `train_losses`, the loss vector the step
+    returns, and `train_params`, every parameter after the step's AdamW update (the trainer's flat buffer, 37 MB).
+    Gradients and the inference outputs are left out: reductions that accumulate with atomics make the gradients of
+    two runs differ by ~1e-4 after one step, and the 10 + W + K training steps in front of the dump amplify that until
+    those arrays no longer correlate between two runs of the same build.  AdamW moves a parameter by at most ~lr per
+    step, so the dumped arrays stay close: two runs of one build with --steps 20 differed by 6e-3 (parameters) and
+    1.3e-2 (losses) relative to their norm (NVIDIA B200, 1000 W power limit)."""
+    import numpy as np
+    torch.cuda.synchronize()
+    host = {k: v.detach().to("cpu", torch.float32).numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    assert total <= DUMP_LIMIT_BYTES, f"--dump-outputs: {total} bytes exceed {DUMP_LIMIT_BYTES}"
+    os.makedirs(path, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 def pooled_sweep(torch, deer_b200, Trainer, dev, use_graph=True, batches=(64, 256, 1024, 4096, 16384, 65536)):

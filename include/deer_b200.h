@@ -159,6 +159,16 @@ int deer_attn_pool_fwd(const float* x, long long xs_b, long long xs_t, const flo
 int deer_attn_pool_bwd(const float* dout, const float* x, long long xs_b, long long xs_t, const float* s, long long ss_b,
                        long long ss_t, const float* mask, const float* wts, float* dx, float* ds, int B, int T, int D,
                        int accumulate, int premask, void* stream);
+/*      pooling over each sample's own frames t < L_b = clamp(lengths[b], 1, T) (lengths [B] int32 / int64 per lengths_i64,
+ *      device memory): softmax and weighted sum over those only; padded rows of x and s are never read, wts is 0 there.
+ *      Backward (wts as written by the forward): ds is 0 at padded rows, and dx (NULL: not produced) is OVERWRITTEN --
+ *      w_t dout at valid rows, 0 at padded rows. */
+int deer_attn_pool_len_fwd(const float* x, long long xs_b, long long xs_t, const float* s, long long ss_b, long long ss_t,
+                           const void* lengths, int lengths_i64, float* out, float* wts, int B, int T, int D,
+                           void* stream);
+int deer_attn_pool_len_bwd(const float* dout, const float* x, long long xs_b, long long xs_t, long long ss_b,
+                           long long ss_t, const void* lengths, int lengths_i64, const float* wts, float* dx, float* ds,
+                           int B, int T, int D, void* stream);
 
 /* ---- layout helpers */
 /* y[t,b,:] = x[b,t,:] (batch-first -> time-major) and the inverse */
@@ -167,6 +177,11 @@ int deer_permute_bt(const float* x, float* y, int B, int T, int D, void* stream)
  *      copies in one pass -- the first nn.LSTM layer's projection operand and its weight-gradient operand
  *      (encoders.py:82-89,380: `self.lstm(enhanced_features)` on a batch_first input) */
 int deer_permute_bt_cast16(const float* x, void* y_fp16, void* y_bf16, int B, int T, int D, int Dp, void* stream);
+/*      the same with per-utterance lengths: rows of frames t >= clamp(lengths[b], 1, T) are written as zeros and their input
+ *      is never read (NaN / Inf padding stays out of the LSTM projection and of dW_ih).  x is [B,T,D], or already
+ *      time-major [T,B,D] when x_time_major != 0.  lengths [B] int32 / int64 (lengths_i64) in device memory. */
+int deer_permute_bt_cast16_len(const float* x, void* y_fp16, void* y_bf16, const void* lengths, int lengths_i64, int B,
+                               int T, int D, int Dp, int x_time_major, void* stream);
 /* y[m,:] = x[m,:] * mask[m]  (text mask, encoders.py:734-735); backward is the same call on dy */
 int deer_rowscale(const float* x, const float* mask, float* y, long long M, int D, void* stream);
 /* Conv1d(k=3,pad=1) lowering on channels-last x [B,T,C]: col [B*T, 3C], tap k holds x[b,t+k-1,:] (zero outside) */
@@ -274,6 +289,15 @@ int deer_lstm_unprep(const float* dwi_il, const float* dwh_il, const float* db_i
                      float* db_hh_rev, int H, int In, void* stream);
 /*      rows g*H+u of src [4H,K] -> rows 4u+g of dst (inverse=0) or back (inverse=1); accumulate!=0 adds into dst */
 int deer_gate_rows_interleave(const float* src, float* dst, int H, int K, int inverse, int accumulate, void* stream);
+/*      per-utterance lengths (nn.LSTM on pack_padded_sequence(x, lengths, batch_first=True, enforce_sorted=False)) on the
+ *      unchanged cluster kernels: between the input projection and the forward recurrence, the i, f and o gates of every
+ *      padded row t >= L_b of pre_il [T,B,2,H,4] (FP16 if pre_fp16, else fp32; 16-byte aligned) are set to -65504.  The
+ *      kernels' sigmoid then gives 2^-60: the state is ~0 at every padded step (the reverse direction starts at L_b - 1 from
+ *      zero, padded outputs <= 2^-83 ~ 1e-25), and with FP16 kept state (DEER_OPT_LSTM_KEEP16 = 1) BPTT produces dpre = 0 exactly
+ *      there, provided dh_out is finite at padded rows.  lengths [B] int32 (lengths_i64 = 0) or int64 (1), device memory,
+ *      clamped to [1, T] by the kernel.  Work scales with the number of padded rows. */
+int deer_lstm_mask_pre(void* pre_il, int pre_fp16, const void* lengths, int lengths_i64, int T, int B, int H,
+                       void* stream);
 
 /* ---- NIG head transform (deer.py:90-98; complete_project.py:399-407). evidence [N,4] -> 7 arrays [N] */
 int deer_nig_head_fwd(const float* evidence, float* mu, float* nu, float* alpha, float* beta, float* aleatoric,

@@ -58,8 +58,11 @@ _PROTOS = {
     "deer_rowdot_bwd": [P, P, P, P, P, P, L, I, P],
     "deer_attn_pool_fwd": [P, L, L, P, L, L, P, P, P, I, I, I, I, P],
     "deer_attn_pool_bwd": [P, P, L, L, P, L, L, P, P, P, P, I, I, I, I, I, P],
+    "deer_attn_pool_len_fwd": [P, L, L, P, L, L, P, I, P, P, I, I, I, P],
+    "deer_attn_pool_len_bwd": [P, P, L, L, L, L, P, I, P, P, P, I, I, I, P],
     "deer_permute_bt": [P, P, I, I, I, P],
     "deer_permute_bt_cast16": [P, P, P, I, I, I, I, P],
+    "deer_permute_bt_cast16_len": [P, P, P, P, I, I, I, I, I, I, P],
     "deer_scorer_bwd": [P, P, P, P, P, P, P, P, L, I, P],
     "deer_rowscale": [P, P, P, L, I, P],
     "deer_im2col3": [P, P, I, I, I, P],
@@ -85,6 +88,7 @@ _PROTOS = {
     "deer_lstm_cluster_xin_mode": [I, I, I],
     "deer_lstm_cluster_fwd_xin": [P, I, P, P, P, P, P, P, P, P, P, I, I, I, P],
     "deer_gate_rows_interleave": [P, P, I, I, I, I, P],
+    "deer_lstm_mask_pre": [P, I, P, I, I, I, I, P],
     "deer_nig_head_fwd": [P, P, P, P, P, P, P, P, L, P],
     "deer_nig_head_bwd": [P, P, P, P, P, P, P, P, P, L, P],
     "deer_nig_loss_stats": [P, P, P, P, P, P, P, P, P, L, I, I, F, P],

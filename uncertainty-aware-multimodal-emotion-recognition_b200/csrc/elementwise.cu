@@ -264,6 +264,69 @@ __global__ void __launch_bounds__(256) permute_bt_cast16_kernel(const float* __r
   }
 }
 
+// ------------------------------------------------------------------ per-utterance lengths (packed-sequence semantics)
+// valid frames of sample b: t < clamp(lengths[b], 1, T) (device lengths are never checked on the host)
+template <typename LenT>
+__device__ __forceinline__ int clamped_length(const LenT* __restrict__ lengths, int b, int T) {
+  const long long L = (long long)lengths[b];
+  return (int)(L < 1 ? 1 : (L > T ? T : L));
+}
+
+// permute_bt_cast16 with the padded frames t >= L_b written as zeros (never read): the 16-bit operand copies of the first
+// LSTM layer then carry no NaN / Inf from the padding into the projection or into dW_ih = dpre^T x (0 * NaN).
+// x_time_major: x is already [T,B,D] (the layer input that needs a gradient went through to_time_major)
+template <typename LenT>
+__global__ void __launch_bounds__(256) permute_bt_cast16_len_kernel(const float* __restrict__ x, __half* __restrict__ y16,
+                                                                    __nv_bfloat16* __restrict__ yb16,
+                                                                    const LenT* __restrict__ lengths, int B, int T, int D,
+                                                                    int Dp, int x_time_major) {
+  DEER_PDL_ENTRY();
+  const int pairs = Dp >> 1;
+  const long long total = (long long)B * T * pairs;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total;
+       i += (long long)gridDim.x * blockDim.x) {
+    const int d = (int)(i % pairs) * 2;
+    const long long r = i / pairs;  // output row = t*B + b
+    const int b = (int)(r % B);
+    const int t = (int)(r / B);
+    float v0 = 0.f, v1 = 0.f;
+    if (t < clamped_length(lengths, b, T)) {
+      const float* src = x + (x_time_major ? r : (long long)b * T + t) * D + d;
+      v0 = d < D ? __ldcs(src) : 0.f;
+      v1 = d + 1 < D ? __ldcs(src + 1) : 0.f;
+    }
+    if (y16) *reinterpret_cast<__half2*>(y16 + r * Dp + d) = __floats2half2_rn(v0, v1);
+    if (yb16) *reinterpret_cast<__nv_bfloat162*>(yb16 + r * Dp + d) = __floats2bfloat162_rn(v0, v1);
+  }
+}
+
+// Gate saturation of the padded rows of the gate-interleaved LSTM pre-activations [T, B, 2 directions, H units, 4 gates]
+// (gate order i, f, g, o): i, f and o of rows t >= L_b are set to -65504 (the most negative finite FP16), so the recurrence
+// kernels' sigmoid gives 2^-60 and the state collapses to ~0 at every padded step -- the reverse direction then starts at
+// L_b - 1 from a zero state, as nn.LSTM does on a packed sequence, and the FP16 gates / cell states kept for BPTT underflow
+// to exactly 0 there (every pre-activation gradient of a padded step is 0).  g is left as it is.
+// grid (B, ny): block (b, y) takes the padded rows L_b + y, L_b + y + ny, ...: the work is that of the padded rows only.
+template <typename LenT, typename Unit>
+__global__ void __launch_bounds__(256) lstm_mask_pre_kernel(Unit* __restrict__ pre, const LenT* __restrict__ lengths,
+                                                            int T, int B, int H) {
+  DEER_PDL_ENTRY();
+  const int b = blockIdx.x;
+  const int units = 2 * H;  // both directions
+  for (int t = clamped_length(lengths, b, T) + blockIdx.y; t < T; t += gridDim.y) {
+    Unit* row = pre + ((long long)t * B + b) * units;
+    for (int u = threadIdx.x; u < units; u += blockDim.x) {
+      Unit v = row[u];
+      if constexpr (sizeof(Unit) == 16) {  // fp32 gates
+        v.x = v.y = v.w = -65504.f;
+      } else {                             // FP16 gates: 0xFBFF = -65504 in the two low halves and the top one
+        v.x = 0xFBFFFBFFu;
+        v.y = (v.y & 0x0000FFFFu) | 0xFBFF0000u;
+      }
+      row[u] = v;
+    }
+  }
+}
+
 __global__ void __launch_bounds__(256) rowscale_kernel(const float* __restrict__ x, const float* __restrict__ mask,
                                                        float* __restrict__ y, long long M, int D) {
   DEER_PDL_ENTRY();
@@ -743,6 +806,46 @@ int deer_permute_bt_cast16(const float* x, void* y_fp16, void* y_bf16, int B, in
   DEER_CHECK_ARG(x && (y_fp16 || y_bf16) && B > 0 && T > 0 && D > 0 && Dp >= D && (Dp & 1) == 0, "permute_bt_cast16: bad args");
   DEER_LAUNCH(permute_bt_cast16_kernel, grid_for((long long)B * T * (Dp / 2)), 256, 0, stream, x,
               reinterpret_cast<__half*>(y_fp16), reinterpret_cast<__nv_bfloat16*>(y_bf16), B, T, D, Dp);
+  return DEER_OK;
+}
+
+int deer_permute_bt_cast16_len(const float* x, void* y_fp16, void* y_bf16, const void* lengths, int lengths_i64, int B,
+                               int T, int D, int Dp, int x_time_major, void* stream) {
+  DEER_CHECK_ARG(x && (y_fp16 || y_bf16) && lengths && B > 0 && T > 0 && D > 0 && Dp >= D && (Dp & 1) == 0,
+                 "permute_bt_cast16_len: bad args");
+  const unsigned grid = grid_for((long long)B * T * (Dp / 2));
+  auto* y16 = reinterpret_cast<__half*>(y_fp16);
+  auto* yb16 = reinterpret_cast<__nv_bfloat16*>(y_bf16);
+  if (lengths_i64)
+    DEER_LAUNCH(permute_bt_cast16_len_kernel<long long>, grid, 256, 0, stream, x, y16, yb16,
+                reinterpret_cast<const long long*>(lengths), B, T, D, Dp, x_time_major);
+  else
+    DEER_LAUNCH(permute_bt_cast16_len_kernel<int>, grid, 256, 0, stream, x, y16, yb16,
+                reinterpret_cast<const int*>(lengths), B, T, D, Dp, x_time_major);
+  return DEER_OK;
+}
+
+int deer_lstm_mask_pre(void* pre, int pre_fp16, const void* lengths, int lengths_i64, int T, int B, int H, void* stream) {
+  DEER_CHECK_ARG(pre && lengths && T > 0 && B > 0 && H > 0 && (reinterpret_cast<uintptr_t>(pre) & 15) == 0,
+                 "lstm_mask_pre: bad args");
+  // up to 8 blocks per sample share its padded rows (one 8 KB FP16 / 16 KB fp32 row per block and trip)
+  const dim3 grid((unsigned)B, (unsigned)(T < 8 ? T : 8));
+  const int threads = 2 * H < 256 ? 2 * H : 256;
+  if (pre_fp16) {
+    if (lengths_i64)
+      DEER_LAUNCH((lstm_mask_pre_kernel<long long, uint2>), grid, threads, 0, stream, reinterpret_cast<uint2*>(pre),
+                  reinterpret_cast<const long long*>(lengths), T, B, H);
+    else
+      DEER_LAUNCH((lstm_mask_pre_kernel<int, uint2>), grid, threads, 0, stream, reinterpret_cast<uint2*>(pre),
+                  reinterpret_cast<const int*>(lengths), T, B, H);
+  } else {
+    if (lengths_i64)
+      DEER_LAUNCH((lstm_mask_pre_kernel<long long, float4>), grid, threads, 0, stream, reinterpret_cast<float4*>(pre),
+                  reinterpret_cast<const long long*>(lengths), T, B, H);
+    else
+      DEER_LAUNCH((lstm_mask_pre_kernel<int, float4>), grid, threads, 0, stream, reinterpret_cast<float4*>(pre),
+                  reinterpret_cast<const int*>(lengths), T, B, H);
+  }
   return DEER_OK;
 }
 

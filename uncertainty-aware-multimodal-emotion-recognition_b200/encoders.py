@@ -40,16 +40,17 @@ def _scorer_pool(x_bt, x_rows, att: nn.Sequential, mask=None):
     return hidden, s
 
 
-def _scorer_and_pool(x, att: nn.Sequential, mask=None, time_major=False, precise=True, x_bf16=None):
+def _scorer_and_pool(x, att: nn.Sequential, mask=None, time_major=False, precise=True, x_bf16=None, lengths=None):
     """Scorer + softmax-over-time pooling of x ([T,B,D] when time_major, else [B,T,D]) as one autograd node
-    (ops.scorer_pool), or as the separate scorer / pooling ops when fusion is switched off."""
+    (ops.scorer_pool), or as the separate scorer / pooling ops when fusion is switched off.  `lengths` (device [B]):
+    pooling over each sample's frames t < L_b only."""
     if ops.scorer_pool_fused():
         return ops.scorer_pool(x, att[0].weight, att[0].bias, att[2].weight, att[2].bias, mask, time_major, precise,
-                               x_bf16)
+                               x_bf16, lengths=lengths)
     _, s = _scorer_pool(None, x, att)
     if time_major:
-        return ops.attn_pool(x.permute(1, 0, 2), s.permute(1, 0), mask)
-    return ops.attn_pool(x, s, mask)
+        return ops.attn_pool(x.permute(1, 0, 2), s.permute(1, 0), mask, lengths)
+    return ops.attn_pool(x, s, mask, lengths)
 
 
 class EnhancedAudioEncoder(nn.Module):
@@ -79,9 +80,12 @@ class EnhancedAudioEncoder(nn.Module):
                 g(f"weight_ih_l{l}_reverse"), g(f"weight_hh_l{l}_reverse"), g(f"bias_ih_l{l}_reverse"),
                 g(f"bias_hh_l{l}_reverse"))
 
-    def lstm_forward(self, features: torch.Tensor, return_bf16: bool = False):
+    def lstm_forward(self, features: torch.Tensor, return_bf16: bool = False, lengths=None):
         """[B,T,84] -> time-major LSTM output [T,B,hidden_dim] (and, on request, the BF16 copy of it that the last
-        layer's recurrence kernel wrote for BPTT: the pooling scorer's weight-gradient GEMM reads it as well)."""
+        layer's recurrence kernel wrote for BPTT: the pooling scorer's weight-gradient GEMM reads it as well).
+        `lengths` [B] (int32 / int64; see ops.sequence_lengths): self.lstm on pack_padded_sequence(features, lengths,
+        batch_first=True, enforce_sorted=False); the output is ~0 (|h| <= 2^-83 ~ 1e-25) at padded frames t >= L_b."""
+        lengths = ops.sequence_lengths(lengths, features.shape[0], features.shape[1], features.device)
         h = features            # batch_first: layer 0 permutes while casting its operands (ops.bilstm_layer)
         h16 = hb16 = None
         nodrop = not (self.training and self.dropout > 0.0)
@@ -93,21 +97,27 @@ class EnhancedAudioEncoder(nn.Module):
             h, h16, hb16 = ops.bilstm_layer(h, *self._layer_weights(l), input_dropout=self.dropout if l > 0 else 0.0,
                                             training=self.training, x_f16=h16,
                                             emit_f16=nodrop and l + 1 < self.num_layers, return_bf16=True,
-                                            x_batch_major=(l == 0))
+                                            x_batch_major=(l == 0), lengths=lengths)
             nodes.append(h.grad_fn)
         # autograd nodes of the layers, first layer first: layer l's weight gradients are complete when node l has run (the
         # data-parallel trainer exchanges the gradients of layers >= 1 beside the BPTT of layer 0)
         self.__dict__["_lstm_bwd_nodes"] = nodes
         return (h, hb16) if return_bf16 else h
 
-    def forward(self, audio_input: torch.Tensor) -> torch.Tensor:
+    def forward(self, audio_input: torch.Tensor, lengths: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """audio_input [B,T,84] frames.  `lengths` [B] (int32 / int64, CUDA or CPU; None: every sample is T frames long):
+        sample b is the utterance audio_input[b, :L_b] and its encoding equals that of the utterance alone -- the LSTM
+        runs as on a packed sequence and the attention softmax covers t < L_b only, so the content of the padded frames
+        (zeros, noise, NaN) does not matter.  CUDA lengths are clamped to [1, T] on the device; CPU lengths outside that
+        range raise."""
         if audio_input.shape[-1] != self.enhanced_features_dim:
             raise NotImplementedError("deer_b200: raw-waveform feature extraction (librosa, CPU) is outside the CUDA hot "
                                       "path; pass pre-extracted 84-D frames [B,T,84]")
         if audio_input.dim() == 2:
             audio_input = audio_input.unsqueeze(1)
-        h_tm, hb16 = self.lstm_forward(audio_input, return_bf16=True)   # [T,B,D]
-        pooled, _ = _scorer_and_pool(h_tm, self.attention, time_major=True, precise=False, x_bf16=hb16)
+        lengths = ops.sequence_lengths(lengths, audio_input.shape[0], audio_input.shape[1], audio_input.device)
+        h_tm, hb16 = self.lstm_forward(audio_input, return_bf16=True, lengths=lengths)   # [T,B,D]
+        pooled, _ = _scorer_and_pool(h_tm, self.attention, time_major=True, precise=False, x_bf16=hb16, lengths=lengths)
         op = self.output_projection
         y = ops.linear(pooled, op[0].weight, op[0].bias, "relu", dropout=self.dropout, training=self.training)
         y = ops.linear(y, op[3].weight, op[3].bias)

@@ -778,11 +778,37 @@ def rowdot(h, w, b):
     return _RowDot.apply(h, w, b)
 
 
+def sequence_lengths(lengths, B: int, T: int, device) -> Optional[torch.Tensor]:
+    """Per-utterance lengths [B] (int32 or int64; sample b is x[b, :L_b], frames t >= L_b are padding whose content does
+    not matter) as the CUDA tensor the length-aware kernels read, in its own dtype (no conversion launch).  A CPU tensor
+    (or a sequence) is validated here -- 1 <= L_b <= T, as pack_padded_sequence requires -- and copied to `device`.  A
+    CUDA tensor is NOT read on the host (that would synchronise and break CUDA-graph capture of a step): the kernels
+    clamp its values to [1, T].  None -> None."""
+    if lengths is None:
+        return None
+    if not torch.is_tensor(lengths):
+        lengths = torch.as_tensor(lengths)
+    if lengths.dtype not in (torch.int32, torch.int64):
+        raise _lib.DeerError(f"deer_b200: lengths must be an int32 or int64 tensor, got {lengths.dtype}")
+    if tuple(lengths.shape) != (B,):
+        raise _lib.DeerError(f"deer_b200: lengths must have shape [{B}], got {tuple(lengths.shape)}")
+    if not lengths.is_cuda:
+        if B > 0 and (int(lengths.min()) < 1 or int(lengths.max()) > T):
+            raise _lib.DeerError(f"deer_b200: lengths must lie in [1, {T}] (got {int(lengths.min())} .. "
+                                 f"{int(lengths.max())})")
+        lengths = lengths.to(device)
+    return lengths.contiguous()
+
+
+def _len_i64(lengths: torch.Tensor) -> int:
+    return int(lengths.dtype == torch.int64)
+
+
 class _AttnPool(torch.autograd.Function):
     """x [B,T,D] (any b/t strides, unit d stride), scores s [B,T] (any strides), mask [B,T] or None."""
 
     @staticmethod
-    def forward(ctx, x, s, mask):
+    def forward(ctx, x, s, mask, lengths=None):
         _req(x, "x"), _req(s, "scores")
         B, T, D = x.shape
         if x.stride(2) != 1:
@@ -790,8 +816,15 @@ class _AttnPool(torch.autograd.Function):
         m = None if mask is None else _req(mask, "mask").contiguous()
         out = torch.empty((B, D), device=x.device, dtype=torch.float32)
         wts = torch.empty((B, T), device=x.device, dtype=torch.float32)
-        call("deer_attn_pool_fwd", ptr(x), x.stride(0), x.stride(1), ptr(s), s.stride(0), s.stride(1), ptr(m), ptr(out),
-             ptr(wts), B, T, D, 0)
+        ctx.lengths = lengths
+        if lengths is not None:
+            if m is not None:
+                raise _lib.DeerError("deer_b200: attn_pool takes a mask or lengths, not both")
+            call("deer_attn_pool_len_fwd", ptr(x), x.stride(0), x.stride(1), ptr(s), s.stride(0), s.stride(1),
+                 lengths.data_ptr(), _len_i64(lengths), ptr(out), ptr(wts), B, T, D)
+        else:
+            call("deer_attn_pool_fwd", ptr(x), x.stride(0), x.stride(1), ptr(s), s.stride(0), s.stride(1), ptr(m),
+                 ptr(out), ptr(wts), B, T, D, 0)
         ctx.save_for_backward(x, s, m, wts)
         ctx.mark_non_differentiable(wts)
         return out, wts
@@ -802,13 +835,19 @@ class _AttnPool(torch.autograd.Function):
         B, T, D = x.shape
         dx = torch.empty_strided(x.shape, x.stride(), device=x.device, dtype=torch.float32)
         ds = torch.empty_strided(s.shape, s.stride(), device=x.device, dtype=torch.float32)
+        if ctx.lengths is not None:
+            call("deer_attn_pool_len_bwd", ptr(dout.contiguous()), ptr(x), x.stride(0), x.stride(1), s.stride(0),
+                 s.stride(1), ctx.lengths.data_ptr(), _len_i64(ctx.lengths), ptr(wts), ptr(dx), ptr(ds), B, T, D)
+            ctx.lengths = None
+            return dx, ds, None, None
         call("deer_attn_pool_bwd", ptr(dout.contiguous()), ptr(x), x.stride(0), x.stride(1), ptr(s), s.stride(0),
              s.stride(1), ptr(m), ptr(wts), ptr(dx), ptr(ds), B, T, D, 0, 0)
-        return dx, ds, None
+        return dx, ds, None, None
 
 
-def attn_pool(x, s, mask=None):
-    return _AttnPool.apply(x, s, mask)
+def attn_pool(x, s, mask=None, lengths=None):
+    """`lengths`: per-utterance lengths (sequence_lengths): softmax and sum over t < L_b only, 0 weight elsewhere."""
+    return _AttnPool.apply(x, s, mask, lengths)
 
 
 class _ScorerPool(torch.autograd.Function):
@@ -820,14 +859,20 @@ class _ScorerPool(torch.autograd.Function):
     input-gradient GEMM accumulates onto it (beta = 1)."""
 
     @staticmethod
-    def forward(ctx, x, w1, b1, w2, b2, mask, time_major, precise=True, x_bf16=None, premask=False):
+    def forward(ctx, x, w1, b1, w2, b2, mask, time_major, precise=True, x_bf16=None, premask=False, lengths=None):
         """x_bf16: optional BF16 copy of x written by its producer (the LSTM recurrence kernel's shadow of h): the B
         operand of dW1 in backward without a cast pass.
         premask: scorer and pooling see x~[b,t] = mask[b,t] x[b,t] (encoders.py:733-735: `token_embeddings *
         attention_mask`) -- applied inside the operand cast and the pooling kernels, the masked copy (50 MB read + write at
-        B = 256) is never materialised.  Batch-major x only; the scorer then runs on the split-precision engine."""
+        B = 256) is never materialised.  Batch-major x only; the scorer then runs on the split-precision engine.
+        lengths: per-utterance lengths [B] (sequence_lengths): the softmax and the weighted sum cover t < L_b only; the
+        scorer still runs on every row, but padded rows get weight 0, ds = 0 and dx = 0, so the scorer's backward GEMMs
+        take nothing from them."""
         x = _req(x, "x").contiguous()
         premask = bool(premask)
+        if lengths is not None and (mask is not None or premask):
+            raise _lib.DeerError("deer_b200: scorer_pool takes a mask or lengths, not both")
+        ctx.lengths = lengths
         if premask and (mask is None or time_major or ctx.needs_input_grad[0] or not (precise and _split_fwd_ok(
                 x.shape[0] * x.shape[1], w1.shape[0], x.shape[2]))):
             raise _lib.DeerError("deer_b200: scorer_pool(premask=True) needs a mask, batch-major x without gradient and a "
@@ -854,7 +899,12 @@ class _ScorerPool(torch.autograd.Function):
         call("deer_rowdot_fwd", ptr(hidden), ptr(w2v), ptr(b2), ptr(sc), M, Hd)
         out = torch.empty((B, D), device=dev, dtype=torch.float32)
         wts = torch.empty((B, T), device=dev, dtype=torch.float32)
-        call("deer_attn_pool_fwd", ptr(x), xs_b, xs_t, ptr(sc), ss_b, ss_t, ptr(m), ptr(out), ptr(wts), B, T, D, int(premask))
+        if lengths is not None:
+            call("deer_attn_pool_len_fwd", ptr(x), xs_b, xs_t, ptr(sc), ss_b, ss_t, lengths.data_ptr(), _len_i64(lengths),
+                 ptr(out), ptr(wts), B, T, D)
+        else:
+            call("deer_attn_pool_fwd", ptr(x), xs_b, xs_t, ptr(sc), ss_b, ss_t, ptr(m), ptr(out), ptr(wts), B, T, D,
+                 int(premask))
         ctx.save_for_backward(x, hidden, sc, m, wts, w1, w2v)
         ctx.premask = premask
         ctx.geom = (B, T, D, M, Hd, xs_b, xs_t, ss_b, ss_t)
@@ -882,8 +932,15 @@ class _ScorerPool(torch.autograd.Function):
         rowterm = bool(need_dx and _state.get("pool_rowterm", True) and _state["engine"] == ENGINE_AUTO and
                        _bwd_engine(M) is None and not (_bwd16_ok(M) and Hd % 8 == 0 and D % 8 == 0) and
                        _lib.tf32_pair_on() and M > 256 and D >= 128 and D % 4 == 0 and Hd >= 64 and Hd % 4 == 0)
-        call("deer_attn_pool_bwd", ptr(doutc), ptr(x), xs_b, xs_t, ptr(sc), ss_b, ss_t, ptr(m), ptr(wts),
-             None if rowterm else ptr(dx), ptr(ds), B, T, D, 0, int(ctx.premask))
+        if ctx.lengths is not None:
+            # dx written as 0 at padded rows (they become the dh the BPTT kernel reads); the GEMMs below add exact zeros
+            # there (ds = 0 -> dh = 0), and the rowterm epilogue's w[b,t] dout[b] is 0 there too
+            call("deer_attn_pool_len_bwd", ptr(doutc), ptr(x), xs_b, xs_t, ss_b, ss_t, ctx.lengths.data_ptr(),
+                 _len_i64(ctx.lengths), ptr(wts), None if rowterm else ptr(dx), ptr(ds), B, T, D)
+            ctx.lengths = None
+        else:
+            call("deer_attn_pool_bwd", ptr(doutc), ptr(x), xs_b, xs_t, ptr(sc), ss_b, ss_t, ptr(m), ptr(wts),
+                 None if rowterm else ptr(dx), ptr(ds), B, T, D, 0, int(ctx.premask))
         dw2, dw2_direct = _acc(pw2, like=w2v)
         db2, db2_direct = _acc(pb2)
         db1, db1_direct = _acc(pb1)
@@ -921,7 +978,7 @@ class _ScorerPool(torch.autograd.Function):
                 gemm(dh, Hd, 1, x, D, 0, dw1, D, Hd, D, M, beta=1.0, engine=_bwd_engine(M))
         ctx.x_bf16 = None
         return (dx if need_dx else None, None if dw1_direct else dw1, None if db1_direct else db1,
-                None if dw2_direct else dw2.view_as(pw2), None if db2_direct else db2, None, None, None, None, None)
+                None if dw2_direct else dw2.view_as(pw2), None if db2_direct else db2, None, None, None, None, None, None)
 
 
 def set_pool_rowterm(on: bool):
@@ -939,16 +996,17 @@ def scorer_pool_fused() -> bool:
     return _state["scorer_pool_fused"]
 
 
-def scorer_pool(x, w1, b1, w2, b2, mask=None, time_major=False, precise=True, x_bf16=None, premask=False):
+def scorer_pool(x, w1, b1, w2, b2, mask=None, time_major=False, precise=True, x_bf16=None, premask=False, lengths=None):
     """(pooled [B,D], attention weights [B,T]) of x [T,B,D] (time_major) or [B,T,D]; see _ScorerPool.  `precise`: the
     scorer's forward GEMM on the split-precision engine (default); False = TF32 (the audio encoder: its pooled output
-    averages 300 highly correlated steps and is dominated by the FP16 recurrence's own 4e-5, measured)."""
+    averages 300 highly correlated steps and is dominated by the FP16 recurrence's own 4e-5, measured).
+    `lengths`: per-utterance lengths (sequence_lengths): pooling over each sample's frames t < L_b only."""
     if premask:
         M = x.shape[0] * x.shape[1]
         if not (precise and _split_fwd_ok(M, w1.shape[0], x.shape[2])):
             # no split-precision engine for this shape (small batches, forced engines): materialise the masked rows
             x, premask = rowscale(x, mask), False
-    return _ScorerPool.apply(x, w1, b1, w2, b2, mask, bool(time_major), bool(precise), x_bf16, bool(premask))
+    return _ScorerPool.apply(x, w1, b1, w2, b2, mask, bool(time_major), bool(precise), x_bf16, bool(premask), lengths)
 
 
 class _RowScale(torch.autograd.Function):
@@ -1142,11 +1200,15 @@ class _BiLSTMLayerCluster(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, wif, whf, bif, bhf, wir, whr, bir, bhr, drop=None, x16_in=None, emit_f16=False,
-                grad_mode=True, batch_major=False):
+                grad_mode=True, batch_major=False, lengths=None):
         """x16_in: FP16 copy of x written by the previous layer's recurrence kernel (skips the cast pass); emit_f16: make
         this layer's kernel write such a copy of h.  Returns (h, h_f16 or an empty tensor).
         batch_major: x is the batch_first input [B,T,In] of the first layer (no gradient): one pass writes its
-        time-major FP16 / BF16 operand copies (no fp32 time-major copy, no cast passes)."""
+        time-major FP16 / BF16 operand copies (no fp32 time-major copy, no cast passes).
+        lengths: per-utterance lengths [B] on the device (sequence_lengths) -- nn.LSTM on a packed sequence.  The input
+        projection then runs as a GEMM (not inside the recurrence kernel), deer_lstm_mask_pre saturates the i / f / o
+        gates of the padded rows of its output, and the recurrence and BPTT kernels run unchanged (DESIGN.md 4.12); the
+        first layer's operand casts write zeros for padded frames."""
         x = _req(x, "x").contiguous()
         if batch_major:
             B, T, In = x.shape
@@ -1157,6 +1219,8 @@ class _BiLSTMLayerCluster(torch.autograd.Function):
         dev = x.device
         keep = grad_mode and any(ctx.needs_input_grad)   # needs_input_grad ignores no_grad(): the caller's mode
         use16 = _state["lstm_gemm16"] and _state["engine"] == ENGINE_AUTO   # a forced engine (tests) is respected
+        if lengths is not None and not use16:
+            raise _lib.DeerError("deer_b200: LSTM lengths need the 16-bit GEMM path (engine AUTO)")
         b_il = torch.empty((2, G), device=dev, dtype=torch.float32)
         w16 = None
         if use16:
@@ -1179,7 +1243,7 @@ class _BiLSTMLayerCluster(torch.autograd.Function):
         pre16 = use16 and _state["lstm_pre16"] and M > 128
         # first layer (In <= 128): the input projection runs INSIDE the recurrence kernel (deer_lstm_cluster_fwd_xin) -- no
         # projection GEMM, no pre-activation tensor
-        xin = bool(use16 and pre16 and drop is None and _state.get("lstm_xin", True) and
+        xin = bool(use16 and pre16 and drop is None and lengths is None and _state.get("lstm_xin", True) and
                    _lib.load().deer_lstm_cluster_xin_mode(B, int(keep), (In + 7) // 8 * 8) > 0)
         pre = None if xin else torch.empty((T, B, 2, G), device=dev, dtype=torch.float16 if pre16 else torch.float32)
         x16 = None
@@ -1199,8 +1263,12 @@ class _BiLSTMLayerCluster(torch.autograd.Function):
             if batch_major:                                   # permute + both 16-bit casts in one pass over x
                 x16 = torch.empty((M, Kp), device=dev, dtype=torch.float16)
                 xb16 = torch.empty((M, Kp), device=dev, dtype=torch.bfloat16) if keep else None
-                call("deer_permute_bt_cast16", ptr(x), x16.data_ptr(), None if xb16 is None else xb16.data_ptr(),
-                     B, T, In, Kp)
+                if lengths is not None:                       # ... zeros for the padded frames
+                    call("deer_permute_bt_cast16_len", ptr(x), x16.data_ptr(), None if xb16 is None else xb16.data_ptr(),
+                         lengths.data_ptr(), _len_i64(lengths), B, T, In, Kp, 0)
+                else:
+                    call("deer_permute_bt_cast16", ptr(x), x16.data_ptr(), None if xb16 is None else xb16.data_ptr(),
+                         B, T, In, Kp)
                 ctx.xdrop_b16 = xb16
             elif drop is not None:                            # dropout + fp16 cast in one pass over x
                 x16 = torch.empty((M, In), device=dev, dtype=torch.float16)
@@ -1221,6 +1289,14 @@ class _BiLSTMLayerCluster(torch.autograd.Function):
             elif (x16_in is not None and x16_in.dtype == torch.float16 and x16_in.numel() == M * In and In % 8 == 0
                   and x16_in.is_contiguous()):
                 x16 = x16_in.view(M, In)                      # the producer kernel's FP16 shadow: no cast pass
+            elif lengths is not None:
+                # FP16 operand and (training) the BF16 one of dW_ih in one pass, zeros for padded frames: a NaN / Inf in the
+                # padding of an input never reaches the projection or dW_ih = dpre^T x
+                x16 = torch.empty((M, Kp), device=dev, dtype=torch.float16)
+                xb16 = torch.empty((M, Kp), device=dev, dtype=torch.bfloat16) if keep else None
+                call("deer_permute_bt_cast16_len", ptr(x), x16.data_ptr(), None if xb16 is None else xb16.data_ptr(),
+                     lengths.data_ptr(), _len_i64(lengths), B, T, In, Kp, 1)
+                ctx.xdrop_b16 = xb16
             else:
                 x16 = cast16(x)                               # [M, Kp] fp16
             assert x16.shape[1] == Kp
@@ -1231,6 +1307,8 @@ class _BiLSTMLayerCluster(torch.autograd.Function):
                 gemm_h16(x16, Kp, 0, w16, Kp, 1, None, 0, M, 2 * G, In, bias=b_il.view(-1), C16=pre, ldc16=2 * G)
             else:
                 gemm_h16(x16, Kp, 0, w16, Kp, 1, pre, 2 * G, M, 2 * G, In, bias=b_il.view(-1))
+            if lengths is not None:
+                call("deer_lstm_mask_pre", pre.data_ptr(), int(pre16), lengths.data_ptr(), _len_i64(lengths), T, B, H)
         else:
             for d in range(2):
                 gemm(x, In, 0, wi_il[d], In, 1, pre.data_ptr() + 4 * G * d, 2 * G, M, G, In, bias=b_il[d])
@@ -1363,7 +1441,7 @@ class _BiLSTMLayerCluster(torch.autograd.Function):
             else:
                 weight_grads()
             r = [None if direct else buf for buf, direct in tg]
-            return dx, r[0], r[2], r[4], r[5], r[1], r[3], r[6], r[7], None, None, None, None, None
+            return dx, r[0], r[2], r[4], r[5], r[1], r[3], r[6], r[7], None, None, None, None, None, None
         for d in range(2):
             gp = dpre.data_ptr() + 4 * G * d
             dwi_il = torch.zeros((G, In), device=dev, dtype=torch.float32)
@@ -1386,13 +1464,16 @@ class _BiLSTMLayerCluster(torch.autograd.Function):
                 dbs.append(None if direct else tgt)
             out.append((None if dwi_direct else dwi, None if dwh_direct else dwh, dbs[0], dbs[1]))
         (dwif, dwhf, dbif, dbhf), (dwir, dwhr, dbir, dbhr) = out
-        return dx, dwif, dwhf, dbif, dbhf, dwir, dwhr, dbir, dbhr, None, None, None, None, None
+        return dx, dwif, dwhf, dbif, dbhf, dwir, dwhr, dbir, dbhr, None, None, None, None, None, None
 
 
 def bilstm_layer(x_tm, wif, whf, bif, bhf, wir, whr, bir, bhr, input_dropout: float = 0.0, training: bool = False,
                  x_f16=None, emit_f16: bool = False, return_f16: bool = False, return_bf16: bool = False,
-                 x_batch_major: bool = False):
+                 x_batch_major: bool = False, lengths=None):
     """engine AUTO/TF32: persistent cluster kernels when H == 256; SIMT: exact-fp32 stepwise; others: see lstm.cu.
+    `lengths`: per-utterance lengths [B] on the device (sequence_lengths): nn.LSTM on
+    pack_padded_sequence(x, lengths, batch_first=True, enforce_sorted=False); h is ~0 (<= 2^-83) at padded rows.  Cluster
+    kernels on the 16-bit GEMM path only: the other engines raise DeerError.
     `x_batch_major`: x_tm is the batch_first [B,T,I] input of the first layer; on the cluster path its time-major 16-bit
     operand copies are written in one pass, elsewhere it is permuted first (ops.to_time_major).
     `input_dropout` (with `training`) applies nn.LSTM's inter-layer dropout to x_tm: fused into the layer's 16-bit
@@ -1401,6 +1482,8 @@ def bilstm_layer(x_tm, wif, whf, bif, bhf, wir, whr, bir, bhr, input_dropout: fl
     (None when the path has none); pass it as `x_f16` to the next layer to skip that layer's operand cast (no-dropout
     case)."""
     cluster = _state["lstm_engine"] in (ENGINE_AUTO, ENGINE_TF32) and whf.shape[1] == 256
+    if lengths is not None and not cluster:
+        raise _lib.DeerError("deer_b200: LSTM lengths are built on the cluster kernels only (H == 256, engine AUTO)")
     drop = None
     bm = False
     if x_batch_major:
@@ -1422,7 +1505,8 @@ def bilstm_layer(x_tm, wif, whf, bif, bhf, wir, whr, bir, bhr, input_dropout: fl
         # (a custom Function's forward always runs with grad mode off: the caller's mode is passed in, so that an
         # inference forward keeps nothing for BPTT and can use the no-keep kernels)
         h, h16, hb16 = _BiLSTMLayerCluster.apply(x_tm, wif, whf, bif, bhf, wir, whr, bir, bhr, drop,
-                                                 x_f16 if drop is None else None, want, torch.is_grad_enabled(), bm)
+                                                 x_f16 if drop is None else None, want, torch.is_grad_enabled(), bm,
+                                                 lengths)
         if return_bf16:     # (h, FP16 copy or None, BF16 copy or None): the 16-bit shadows the recurrence kernel wrote
             return h, (h16 if h16.numel() else None), (hb16 if hb16.numel() else None)
         return (h, h16 if h16.numel() else None) if return_f16 else h

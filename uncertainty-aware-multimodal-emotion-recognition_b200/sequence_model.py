@@ -32,7 +32,10 @@ class SequenceDEERModel(nn.Module):
         self.loss_fn = MultiTaskDEERLoss()
 
     def forward(self, audio, video=None, text=None, attention_mask: Optional[torch.Tensor] = None,
-                linguistic_features: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
+                linguistic_features: Optional[torch.Tensor] = None,
+                audio_lengths: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
+        """`audio_lengths` [B] (int32 / int64; also read from the batch dict key "audio_lengths"): frames of each audio
+        utterance, see EnhancedAudioEncoder.forward.  None: every sample has all T frames."""
         if isinstance(audio, dict):
             d = audio
             audio = d.get("audio", d.get("audio_features"))
@@ -40,6 +43,7 @@ class SequenceDEERModel(nn.Module):
             text = d.get("text", d.get("text_features"))
             attention_mask = d.get("attention_mask", attention_mask)
             linguistic_features = d.get("linguistic_features", linguistic_features)
+            audio_lengths = d.get("audio_lengths", audio_lengths)
         ops.begin_step()
         # training: up to 512 samples the recurrence is ONE wave of clusters; beyond that the second wave of the
         # (gate / cell storing) kernels competes with the side work for SMs.  Inference forwards (no stores for BPTT,
@@ -58,7 +62,7 @@ class SequenceDEERModel(nn.Module):
             side.wait_stream(main)
             ops.mark("step_start")
             with torch.cuda.stream(side):
-                a = ops.mark_tensor(self.audio_encoder(ops.mark_tensor(audio, "audio_in")), "audio_out")
+                a = ops.mark_tensor(self.audio_encoder(ops.mark_tensor(audio, "audio_in"), audio_lengths), "audio_out")
             tside = self._branch_stream("text", 0) if ops.text_stream_enabled() else None
             if tside is not None:
                 # the text encoder (one scorer GEMM, small kernels) on a third stream: with the first LSTM layer's input
@@ -82,7 +86,7 @@ class SequenceDEERModel(nn.Module):
             a.record_stream(main)
             ops.mark("joined")
         else:
-            a = self.audio_encoder(audio)
+            a = self.audio_encoder(audio, audio_lengths)
             v = self.video_encoder(video)
             t = self.text_encoder(text, attention_mask, linguistic_features)
         if chain.enabled() and a.is_cuda and chain.supported(self.fusion, self.deer, a, v, t):

@@ -162,7 +162,9 @@ int deer_attn_pool_bwd(const float* dout, const float* x, long long xs_b, long l
 /*      pooling over each sample's own frames t < L_b = clamp(lengths[b], 1, T) (lengths [B] int32 / int64 per lengths_i64,
  *      device memory): softmax and weighted sum over those only; padded rows of x and s are never read, wts is 0 there.
  *      Backward (wts as written by the forward): ds is 0 at padded rows, and dx (NULL: not produced) is OVERWRITTEN --
- *      w_t dout at valid rows, 0 at padded rows. */
+ *      w_t dout at valid rows, 0 at padded rows.  These run the kernels of deer_attn_pool_fwd / _bwd (their
+ *      length-bounded instantiations): with every length equal to T they write the same bits as those entries do
+ *      without a mask. */
 int deer_attn_pool_len_fwd(const float* x, long long xs_b, long long xs_t, const float* s, long long ss_b, long long ss_t,
                            const void* lengths, int lengths_i64, float* out, float* wts, int B, int T, int D,
                            void* stream);
@@ -179,7 +181,8 @@ int deer_permute_bt(const float* x, float* y, int B, int T, int D, void* stream)
 int deer_permute_bt_cast16(const float* x, void* y_fp16, void* y_bf16, int B, int T, int D, int Dp, void* stream);
 /*      the same with per-utterance lengths: rows of frames t >= clamp(lengths[b], 1, T) are written as zeros and their input
  *      is never read (NaN / Inf padding stays out of the LSTM projection and of dW_ih).  x is [B,T,D], or already
- *      time-major [T,B,D] when x_time_major != 0.  lengths [B] int32 / int64 (lengths_i64) in device memory. */
+ *      time-major [T,B,D] when x_time_major != 0.  lengths [B] int32 / int64 (lengths_i64) in device memory.  The kernel
+ *      of deer_permute_bt_cast16, length-bounded. */
 int deer_permute_bt_cast16_len(const float* x, void* y_fp16, void* y_bf16, const void* lengths, int lengths_i64, int B,
                                int T, int D, int Dp, int x_time_major, void* stream);
 /* y[m,:] = x[m,:] * mask[m]  (text mask, encoders.py:734-735); backward is the same call on dy */

@@ -187,6 +187,48 @@ def test_full_lengths_equal_no_lengths(B, T):
                 assert_grad_cosine(g1[n], g0[n], n, 0.9999)
 
 
+@pytest.mark.parametrize("dtype", [torch.int32, torch.int64])
+def test_length_entries_at_full_length_equal_plain_entries(dtype):
+    """The length entries launch the pooling and permute-cast kernels of their plain counterparts: with every length
+    equal to T they write the same bits (B = 256, T = 300, the audio encoder's pooling and layer-0 operand shapes)."""
+    B, T, D, In, Kp = 256, 300, 512, 84, 88
+    g = torch.Generator(device=DEV).manual_seed(12)
+    x = torch.randn(T, B, D, device=DEV, generator=g)             # time-major, as the audio encoder pools it
+    s = torch.randn(T, B, device=DEV, generator=g)
+    dout = torch.randn(B, D, device=DEV, generator=g)
+    xs_b, xs_t, ss_b, ss_t = D, B * D, 1, B
+    full = torch.full((B,), T, dtype=dtype, device=DEV)
+    i64 = int(dtype == torch.int64)
+    res = []
+    for lens in (None, full):
+        out, wts = torch.empty(B, D, device=DEV), torch.empty(B, T, device=DEV)
+        dx, ds = torch.empty_like(x), torch.empty_like(s)
+        if lens is None:
+            ops.call("deer_attn_pool_fwd", ops.ptr(x), xs_b, xs_t, ops.ptr(s), ss_b, ss_t, None, ops.ptr(out),
+                     ops.ptr(wts), B, T, D, 0)
+            ops.call("deer_attn_pool_bwd", ops.ptr(dout), ops.ptr(x), xs_b, xs_t, ops.ptr(s), ss_b, ss_t, None,
+                     ops.ptr(wts), ops.ptr(dx), ops.ptr(ds), B, T, D, 0, 0)
+        else:
+            ops.call("deer_attn_pool_len_fwd", ops.ptr(x), xs_b, xs_t, ops.ptr(s), ss_b, ss_t, lens.data_ptr(), i64,
+                     ops.ptr(out), ops.ptr(wts), B, T, D)
+            ops.call("deer_attn_pool_len_bwd", ops.ptr(dout), ops.ptr(x), xs_b, xs_t, ss_b, ss_t, lens.data_ptr(), i64,
+                     ops.ptr(wts), ops.ptr(dx), ops.ptr(ds), B, T, D)
+        res.append({"out": out, "wts": wts, "dx": dx, "ds": ds})
+    xa = torch.randn(B, T, In, device=DEV, generator=g)            # batch-first layer-0 input
+    for r, lens in zip(res, (None, full)):
+        y16 = torch.empty(T * B, Kp, device=DEV, dtype=torch.float16)
+        yb16 = torch.empty(T * B, Kp, device=DEV, dtype=torch.bfloat16)
+        if lens is None:
+            ops.call("deer_permute_bt_cast16", ops.ptr(xa), y16.data_ptr(), yb16.data_ptr(), B, T, In, Kp)
+        else:
+            ops.call("deer_permute_bt_cast16_len", ops.ptr(xa), y16.data_ptr(), yb16.data_ptr(), lens.data_ptr(), i64,
+                     B, T, In, Kp, 0)
+        r.update(y16=y16, yb16=yb16)
+    torch.cuda.synchronize()
+    for k in res[0]:
+        assert torch.equal(res[0][k], res[1][k]), k
+
+
 def test_device_lengths_are_clamped_and_dtypes_agree():
     B, T = 37, 24
     enc, _ = encoder(2)

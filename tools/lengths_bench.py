@@ -8,7 +8,8 @@ Training step (B = 256, T = 300, the data-parallel trainer's whole step captured
   ragged   -- audio_lengths uniform in [75, 300]
 Inference (B = 1024, eval forward captured as a CUDA graph): without / with ragged lengths.
 Kernels (CUDA events over 200 launches each, B = 256, T = 300): attention pooling forward / backward dense vs
-length-aware on the ragged lengths, with the bytes each reads; the saturation pass on the FP16 pre-activations.
+length-aware on the ragged lengths, with the bytes each reads; the layer-0 permute + 16-bit cast dense vs length-aware;
+the saturation pass on the FP16 pre-activations.
 Prints one JSON object (GPU name and power limit included); --out also writes it to FILE."""
 from __future__ import annotations
 
@@ -131,6 +132,13 @@ def main():
         "pool_bwd_len": lambda: L.deer_attn_pool_len_bwd(p(dout), p(x), xs_b, xs_t, ss_b, ss_t, p(lens), 0, p(wts),
                                                          p(dx), p(ds), B, T, D, st()),
     }
+    In, Kp = 84, 88                                      # the audio encoder's layer-0 input and its padded K
+    xa = torch.randn(B, T, In, device=dev)
+    xa16 = torch.empty(T * B, Kp, device=dev, dtype=torch.float16)
+    xab16 = torch.empty(T * B, Kp, device=dev, dtype=torch.bfloat16)
+    kern["permute_cast16_dense"] = lambda: L.deer_permute_bt_cast16(p(xa), p(xa16), p(xab16), B, T, In, Kp, st())
+    kern["permute_cast16_len"] = lambda: L.deer_permute_bt_cast16_len(p(xa), p(xa16), p(xab16), p(lens), 0, B, T, In,
+                                                                      Kp, 0, st())
     pre16 = torch.empty(T, B, 2, 4 * H, device=dev, dtype=torch.float16)
     kern["mask_pre_fp16_ragged"] = lambda: L.deer_lstm_mask_pre(p(pre16), 1, p(lens), 0, T, B, H, st())
     full = batches["full"]["audio_lengths"]

@@ -93,6 +93,13 @@ __device__ __forceinline__ float block_sum(float v, float* red) {
   return r;
 }
 
+// per-utterance lengths (packed-sequence semantics): sample b's valid frames are t < clamp(lengths[b], 1, T), lengths
+// [B] int32 or int64 (i64 != 0) in device memory, never checked on the host
+__device__ __forceinline__ int seq_length(const void* lengths, int i64, int b, int T) {
+  const long long L = i64 ? static_cast<const long long*>(lengths)[b] : static_cast<const int*>(lengths)[b];
+  return (int)(L < 1 ? 1 : (L > T ? T : L));
+}
+
 // accurate fp32 sigmoid / tanh on the MUFU pipe (ex2 + rcp): |rel err| ~ 2 ulp
 __device__ __forceinline__ float sigmoid_f(float x) { return __fdividef(1.f, 1.f + __expf(-x)); }
 __device__ __forceinline__ float tanh_f(float x) {

@@ -804,6 +804,26 @@ def _len_i64(lengths: torch.Tensor) -> int:
     return int(lengths.dtype == torch.int64)
 
 
+def _pool_fwd(x, xs_b, xs_t, s, ss_b, ss_t, m, lengths, out, wts, B, T, D, premask=False):
+    """Attention pooling forward over each sample's frames t < L_b (lengths) or over all T (mask m / premask)."""
+    if lengths is not None:
+        call("deer_attn_pool_len_fwd", ptr(x), xs_b, xs_t, ptr(s), ss_b, ss_t, lengths.data_ptr(), _len_i64(lengths),
+             ptr(out), ptr(wts), B, T, D)
+    else:
+        call("deer_attn_pool_fwd", ptr(x), xs_b, xs_t, ptr(s), ss_b, ss_t, ptr(m), ptr(out), ptr(wts), B, T, D,
+             int(premask))
+
+
+def _pool_bwd(dout, x, xs_b, xs_t, s, ss_b, ss_t, m, lengths, wts, dx, ds, B, T, D, premask=False):
+    """Attention pooling backward, dx overwritten (None: not produced); with lengths dx and ds are 0 at padded rows."""
+    if lengths is not None:
+        call("deer_attn_pool_len_bwd", ptr(dout), ptr(x), xs_b, xs_t, ss_b, ss_t, lengths.data_ptr(), _len_i64(lengths),
+             ptr(wts), ptr(dx), ptr(ds), B, T, D)
+    else:
+        call("deer_attn_pool_bwd", ptr(dout), ptr(x), xs_b, xs_t, ptr(s), ss_b, ss_t, ptr(m), ptr(wts), ptr(dx), ptr(ds),
+             B, T, D, 0, int(premask))
+
+
 class _AttnPool(torch.autograd.Function):
     """x [B,T,D] (any b/t strides, unit d stride), scores s [B,T] (any strides), mask [B,T] or None."""
 
@@ -814,17 +834,12 @@ class _AttnPool(torch.autograd.Function):
         if x.stride(2) != 1:
             x = x.contiguous()
         m = None if mask is None else _req(mask, "mask").contiguous()
+        if lengths is not None and m is not None:
+            raise _lib.DeerError("deer_b200: attn_pool takes a mask or lengths, not both")
         out = torch.empty((B, D), device=x.device, dtype=torch.float32)
         wts = torch.empty((B, T), device=x.device, dtype=torch.float32)
         ctx.lengths = lengths
-        if lengths is not None:
-            if m is not None:
-                raise _lib.DeerError("deer_b200: attn_pool takes a mask or lengths, not both")
-            call("deer_attn_pool_len_fwd", ptr(x), x.stride(0), x.stride(1), ptr(s), s.stride(0), s.stride(1),
-                 lengths.data_ptr(), _len_i64(lengths), ptr(out), ptr(wts), B, T, D)
-        else:
-            call("deer_attn_pool_fwd", ptr(x), x.stride(0), x.stride(1), ptr(s), s.stride(0), s.stride(1), ptr(m),
-                 ptr(out), ptr(wts), B, T, D, 0)
+        _pool_fwd(x, x.stride(0), x.stride(1), s, s.stride(0), s.stride(1), m, lengths, out, wts, B, T, D)
         ctx.save_for_backward(x, s, m, wts)
         ctx.mark_non_differentiable(wts)
         return out, wts
@@ -835,13 +850,9 @@ class _AttnPool(torch.autograd.Function):
         B, T, D = x.shape
         dx = torch.empty_strided(x.shape, x.stride(), device=x.device, dtype=torch.float32)
         ds = torch.empty_strided(s.shape, s.stride(), device=x.device, dtype=torch.float32)
-        if ctx.lengths is not None:
-            call("deer_attn_pool_len_bwd", ptr(dout.contiguous()), ptr(x), x.stride(0), x.stride(1), s.stride(0),
-                 s.stride(1), ctx.lengths.data_ptr(), _len_i64(ctx.lengths), ptr(wts), ptr(dx), ptr(ds), B, T, D)
-            ctx.lengths = None
-            return dx, ds, None, None
-        call("deer_attn_pool_bwd", ptr(dout.contiguous()), ptr(x), x.stride(0), x.stride(1), ptr(s), s.stride(0),
-             s.stride(1), ptr(m), ptr(wts), ptr(dx), ptr(ds), B, T, D, 0, 0)
+        _pool_bwd(dout.contiguous(), x, x.stride(0), x.stride(1), s, s.stride(0), s.stride(1), m, ctx.lengths, wts, dx, ds,
+                  B, T, D)
+        ctx.lengths = None
         return dx, ds, None, None
 
 
@@ -899,12 +910,7 @@ class _ScorerPool(torch.autograd.Function):
         call("deer_rowdot_fwd", ptr(hidden), ptr(w2v), ptr(b2), ptr(sc), M, Hd)
         out = torch.empty((B, D), device=dev, dtype=torch.float32)
         wts = torch.empty((B, T), device=dev, dtype=torch.float32)
-        if lengths is not None:
-            call("deer_attn_pool_len_fwd", ptr(x), xs_b, xs_t, ptr(sc), ss_b, ss_t, lengths.data_ptr(), _len_i64(lengths),
-                 ptr(out), ptr(wts), B, T, D)
-        else:
-            call("deer_attn_pool_fwd", ptr(x), xs_b, xs_t, ptr(sc), ss_b, ss_t, ptr(m), ptr(out), ptr(wts), B, T, D,
-                 int(premask))
+        _pool_fwd(x, xs_b, xs_t, sc, ss_b, ss_t, m, lengths, out, wts, B, T, D, premask)
         ctx.save_for_backward(x, hidden, sc, m, wts, w1, w2v)
         ctx.premask = premask
         ctx.geom = (B, T, D, M, Hd, xs_b, xs_t, ss_b, ss_t)
@@ -932,15 +938,11 @@ class _ScorerPool(torch.autograd.Function):
         rowterm = bool(need_dx and _state.get("pool_rowterm", True) and _state["engine"] == ENGINE_AUTO and
                        _bwd_engine(M) is None and not (_bwd16_ok(M) and Hd % 8 == 0 and D % 8 == 0) and
                        _lib.tf32_pair_on() and M > 256 and D >= 128 and D % 4 == 0 and Hd >= 64 and Hd % 4 == 0)
-        if ctx.lengths is not None:
-            # dx written as 0 at padded rows (they become the dh the BPTT kernel reads); the GEMMs below add exact zeros
-            # there (ds = 0 -> dh = 0), and the rowterm epilogue's w[b,t] dout[b] is 0 there too
-            call("deer_attn_pool_len_bwd", ptr(doutc), ptr(x), xs_b, xs_t, ss_b, ss_t, ctx.lengths.data_ptr(),
-                 _len_i64(ctx.lengths), ptr(wts), None if rowterm else ptr(dx), ptr(ds), B, T, D)
-            ctx.lengths = None
-        else:
-            call("deer_attn_pool_bwd", ptr(doutc), ptr(x), xs_b, xs_t, ptr(sc), ss_b, ss_t, ptr(m), ptr(wts),
-                 None if rowterm else ptr(dx), ptr(ds), B, T, D, 0, int(ctx.premask))
+        # with lengths dx is written as 0 at padded rows (they become the dh the BPTT kernel reads); the GEMMs below add
+        # exact zeros there (ds = 0 -> dh = 0), and the rowterm epilogue's w[b,t] dout[b] is 0 there too
+        _pool_bwd(doutc, x, xs_b, xs_t, sc, ss_b, ss_t, m, ctx.lengths, wts, None if rowterm else dx, ds, B, T, D,
+                  ctx.premask)
+        ctx.lengths = None
         dw2, dw2_direct = _acc(pw2, like=w2v)
         db2, db2_direct = _acc(pb2)
         db1, db1_direct = _acc(pb1)
@@ -1260,12 +1262,17 @@ class _BiLSTMLayerCluster(torch.autograd.Function):
             raise _lib.DeerError("deer_b200: batch_major LSTM input needs the 16-bit GEMM path, no input dropout and an "
                                  "input without gradient")
         if use16:
-            if batch_major:                                   # permute + both 16-bit casts in one pass over x
+            shadow16 = (x16_in is not None and x16_in.dtype == torch.float16 and x16_in.numel() == M * In and In % 8 == 0
+                        and x16_in.is_contiguous())
+            if batch_major or (lengths is not None and drop is None and not shadow16):
+                # (permute +) both 16-bit casts in one pass over x: the FP16 operand and (training) the BF16 one of dW_ih;
+                # with lengths, zeros for padded frames: a NaN / Inf in the padding of an input never reaches the
+                # projection or dW_ih = dpre^T x
                 x16 = torch.empty((M, Kp), device=dev, dtype=torch.float16)
                 xb16 = torch.empty((M, Kp), device=dev, dtype=torch.bfloat16) if keep else None
-                if lengths is not None:                       # ... zeros for the padded frames
+                if lengths is not None:
                     call("deer_permute_bt_cast16_len", ptr(x), x16.data_ptr(), None if xb16 is None else xb16.data_ptr(),
-                         lengths.data_ptr(), _len_i64(lengths), B, T, In, Kp, 0)
+                         lengths.data_ptr(), _len_i64(lengths), B, T, In, Kp, int(not batch_major))
                 else:
                     call("deer_permute_bt_cast16", ptr(x), x16.data_ptr(), None if xb16 is None else xb16.data_ptr(),
                          B, T, In, Kp)
@@ -1286,17 +1293,8 @@ class _BiLSTMLayerCluster(torch.autograd.Function):
                      None if kmask is None else kmask.data_ptr())
                 ctx.xdrop_b16 = xdrop_b16
                 ctx.drop_mask = kmask
-            elif (x16_in is not None and x16_in.dtype == torch.float16 and x16_in.numel() == M * In and In % 8 == 0
-                  and x16_in.is_contiguous()):
+            elif shadow16:
                 x16 = x16_in.view(M, In)                      # the producer kernel's FP16 shadow: no cast pass
-            elif lengths is not None:
-                # FP16 operand and (training) the BF16 one of dW_ih in one pass, zeros for padded frames: a NaN / Inf in the
-                # padding of an input never reaches the projection or dW_ih = dpre^T x
-                x16 = torch.empty((M, Kp), device=dev, dtype=torch.float16)
-                xb16 = torch.empty((M, Kp), device=dev, dtype=torch.bfloat16) if keep else None
-                call("deer_permute_bt_cast16_len", ptr(x), x16.data_ptr(), None if xb16 is None else xb16.data_ptr(),
-                     lengths.data_ptr(), _len_i64(lengths), B, T, In, Kp, 1)
-                ctx.xdrop_b16 = xb16
             else:
                 x16 = cast16(x)                               # [M, Kp] fp16
             assert x16.shape[1] == Kp

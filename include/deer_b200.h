@@ -187,6 +187,11 @@ int deer_permute_bt_cast16_len(const float* x, void* y_fp16, void* y_bf16, const
                                int T, int D, int Dp, int x_time_major, void* stream);
 /* y[m,:] = x[m,:] * mask[m]  (text mask, encoders.py:734-735); backward is the same call on dy */
 int deer_rowscale(const float* x, const float* mask, float* y, long long M, int D, void* stream);
+/*      the same kernel with the mask taken from per-utterance lengths: x, y [B,T,D], y = x at frames t < clamp(lengths[b], 1, T)
+ *      and y = 0 at padded frames, whose rows of x are never read (NaN / Inf padding is not carried).  The masked copy of the
+ *      video encoder's input in front of spatial_projection (encoders.py:531-533, so dW = dz^T x takes no 0 * NaN) and of
+ *      the im2col Conv1d's input and input gradient; backward is the same call on dy. */
+int deer_rowscale_len(const float* x, float* y, const void* lengths, int lengths_i64, int B, int T, int D, void* stream);
 /* Conv1d(k=3,pad=1) lowering on channels-last x [B,T,C]: col [B*T, 3C], tap k holds x[b,t+k-1,:] (zero outside) */
 int deer_im2col3(const float* x, float* col, int B, int T, int C, void* stream);
 int deer_col2im3(const float* dcol, float* dx, int B, int T, int C, void* stream);
@@ -203,6 +208,14 @@ int deer_rows_pad(const float* src, float* dst, int B, int T, int C, int lead, i
 int deer_rows_pad_fused(const float* src, float* dst, void* hi, void* lo, int B, int T, int C, int lead, int tail, int dir,
                         float drop_p, unsigned long long seed, unsigned long long offset, const unsigned long long* step_ptr,
                         void* stream);
+/*      the same with per-utterance lengths (nn.Conv1d(padding=1) on each clip x[b, :L_b] alone, L_b = clamp(lengths[b], 1, T)):
+ *      frames t >= L_b are treated as pad rows.  dir 0 writes them as zeros in xp and in the hi / lo copies and does not
+ *      read them, so the tap at t = L_b reads 0; dir 1 writes dx = 0 there (dx_p row L_b holds dy[L_b - 1] W's tap, which
+ *      must not reach the padded rows).  The kernel of deer_rows_pad_fused, length-bounded: with every length equal to T
+ *      it writes the same bits. */
+int deer_rows_pad_fused_len(const float* src, float* dst, void* hi, void* lo, const void* lengths, int lengths_i64, int B,
+                            int T, int C, int lead, int tail, int dir, float drop_p, unsigned long long seed,
+                            unsigned long long offset, const unsigned long long* step_ptr, void* stream);
 /*      backward entry of the same convolution: dy [B,T,C] -> dy_big [B*(T+1), C] (a zero row behind every sample) and the
  *      bias gradient colsum[c] += sum over rows of dy[., c] (nn.Conv1d.bias, encoders.py:450-459) in ONE pass over dy */
 int deer_rows_pad_colsum(const float* src, float* dst, float* colsum, int B, int T, int C, void* stream);
@@ -223,6 +236,24 @@ int deer_bn_relu_fwd(const float* x, const float* mean, const float* var, const 
 int deer_bn_relu_bwd(const float* dy, const float* x, const float* y, const float* mean, const float* var,
                      const float* gamma, float* dx, float* dgamma, float* dbeta, float* scratch, long long M, int C,
                      float eps, int batch_stats, void* stream);
+/*      the same over per-utterance lengths: x, y, dy, dx are [B,T,C] and only the frames t < clamp(lengths[b], 1, T) are
+ *      rows of the batch -- nn.BatchNorm1d applied to the valid frames packed into one [N, C] batch, N = sum_b L_b.
+ *      N is counted on the device and carried in the statistics: stats is [2C+1] (mean, biased var, N), zeroed and
+ *      written by deer_bn_stats_len; deer_bn_update_running_len reads N there (unbiased factor N/(N-1) when N > 1;
+ *      num_batches_tracked += 1).  Padded rows are never read: the forward writes y = 0 and the backward dx = 0 there,
+ *      and the backward's reductions skip them.  With batch_stats, mean must be that stats buffer and var = mean + C
+ *      (1/N is read at mean[2C]).  These run the kernels of the entries above, length-bounded: with every length equal to
+ *      T the forward writes the same bits. */
+int deer_bn_stats_len(const float* x, float* stats, const void* lengths, int lengths_i64, int B, int T, int C,
+                      void* stream);
+int deer_bn_update_running_len(const float* stats, float* running_mean, float* running_var,
+                               long long* num_batches_tracked /* int64 counter or NULL */, int C, float momentum,
+                               void* stream);
+int deer_bn_relu_fwd_len(const float* x, const float* mean, const float* var, const float* gamma, const float* beta,
+                         float* y, const void* lengths, int lengths_i64, int B, int T, int C, float eps, void* stream);
+int deer_bn_relu_bwd_len(const float* dy, const float* x, const float* y, const float* mean, const float* var,
+                         const float* gamma, float* dx, float* dgamma, float* dbeta, float* scratch, const void* lengths,
+                         int lengths_i64, int B, int T, int C, float eps, int batch_stats, void* stream);
 
 /* ---- 2-token multi-head self attention core (fusion.py:293-298,328-332): qkv [B,2,3E] packed (q|k|v) after in_proj,
  *      ctx [B,2,E] before out_proj, attw [B,2,2] head-averaged weights. */

@@ -1,15 +1,21 @@
-"""Cost of per-utterance audio lengths, measured in one process, alternating the configurations on the same GPU.
+"""Cost of per-utterance audio and video lengths, measured in one process, alternating the configurations on the same GPU.
 
     python tools/lengths_bench.py [--steps 40] [--rounds 5] [--out FILE]
 
-Training step (B = 256, T = 300, the data-parallel trainer's whole step captured as a CUDA graph, inputs resident):
-  default  -- no lengths (bench.py's workload)
-  full     -- audio_lengths = T for every sample (layer 0 through the projection GEMM + saturation pass)
-  ragged   -- audio_lengths uniform in [75, 300]
-Inference (B = 1024, eval forward captured as a CUDA graph): without / with ragged lengths.
-Kernels (CUDA events over 200 launches each, B = 256, T = 300): attention pooling forward / backward dense vs
+Training step (B = 256, audio T = 300, video T = 50, the data-parallel trainer's whole step captured as a CUDA graph,
+inputs resident):
+  default       -- no lengths (bench.py's workload)
+  full          -- audio_lengths = T for every sample (layer 0 through the projection GEMM + saturation pass)
+  ragged        -- audio_lengths uniform in [75, 300]
+  video_full    -- video_lengths = 50 for every clip
+  video_ragged  -- video_lengths uniform in [12, 50]
+  both_ragged   -- audio and video lengths ragged as above
+Inference (B = 1024, eval forward captured as a CUDA graph): without lengths, with ragged audio / ragged video lengths.
+Kernels (CUDA events over 200 launches each, B = 256): at T = 300 attention pooling forward / backward dense vs
 length-aware on the ragged lengths, with the bytes each reads; the layer-0 permute + 16-bit cast dense vs length-aware;
-the saturation pass on the FP16 pre-activations.
+the saturation pass on the FP16 pre-activations.  At T = 50, C = 512 (the video encoder): BatchNorm statistics, BN+ReLU
+forward and backward, the Conv1d padding pass (forward with the FP16 hi / lo split, backward un-pad) plain vs
+length-aware on ragged video lengths, and the input masking copy.
 Prints one JSON object (GPU name and power limit included); --out also writes it to FILE."""
 from __future__ import annotations
 
@@ -23,6 +29,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
 TRAIN_B, INFER_B, T = 256, 1024, 300
+TV, CV, DV = 50, 512, 256          # video frames, video encoder width, frame features
 
 
 def gpu_info(torch):
@@ -57,6 +64,9 @@ def main():
     def ragged(B):
         return torch.randint(75, T + 1, (B,), generator=gen, dtype=torch.int32).to(dev)
 
+    def vragged(B):
+        return torch.randint(TV // 4, TV + 1, (B,), generator=gen, dtype=torch.int32).to(dev)
+
     def timed(fn, n):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
@@ -75,11 +85,17 @@ def main():
     trainer = DEERDataParallelTrainer(model, learning_rate=1e-4, weight_decay=1e-5, gradient_clip=1.0)
     base = synth_batch(TRAIN_B, dev, gen)
     batches = {"default": base, "full": dict(base, audio_lengths=torch.full((TRAIN_B,), T, dtype=torch.int32, device=dev)),
-               "ragged": dict(base, audio_lengths=ragged(TRAIN_B))}
+               "ragged": dict(base, audio_lengths=ragged(TRAIN_B)),
+               "video_full": dict(base, video_lengths=torch.full((TRAIN_B,), TV, dtype=torch.int32, device=dev)),
+               "video_ragged": dict(base, video_lengths=vragged(TRAIN_B))}
+    batches["both_ragged"] = dict(base, audio_lengths=batches["ragged"]["audio_lengths"],
+                                  video_lengths=batches["video_ragged"]["video_lengths"])
     launches, replays = {}, {}
+    for b in batches.values():      # the zeroed scratch arena grows over the first steps: count launches once it is settled
+        for _ in range(3):
+            trainer.train_step(b)
+    torch.cuda.synchronize()
     for name, b in batches.items():
-        trainer.train_step(b)
-        torch.cuda.synchronize()
         l0 = _lib.launch_count()
         trainer.train_step(b)
         launches[name] = _lib.launch_count() - l0
@@ -98,7 +114,8 @@ def main():
     keys = ("audio_features", "video_features", "text_features", "attention_mask", "linguistic_features")
     ilen = ragged(INFER_B)
     ireplay = {"default": capture_forward(model, *[ib[k] for k in keys])[0],
-               "ragged": capture_forward(model, *[ib[k] for k in keys], audio_lengths=ilen)[0]}
+               "ragged": capture_forward(model, *[ib[k] for k in keys], audio_lengths=ilen)[0],
+               "video_ragged": capture_forward(model, *[ib[k] for k in keys], video_lengths=vragged(INFER_B))[0]}
     infer_ms = {k: [] for k in ireplay}
     for _ in range(args.rounds):
         for name, fn in ireplay.items():
@@ -148,6 +165,49 @@ def main():
         assert fn() == 0, name
         torch.cuda.synchronize()
         kern_us[name] = round(timed(fn, 200) * 1e3, 2)
+
+    # ------------------------------------------------------------------ video encoder kernels at B = 256, T = 50, C = 512
+    vlens = batches["video_ragged"]["video_lengths"]
+    M = B * TV
+    xv = torch.randn(B, TV, CV, device=dev)
+    yv, dyv, dxv = torch.empty_like(xv), torch.randn(B, TV, CV, device=dev), torch.empty_like(xv)
+    gam, bet = torch.rand(CV, device=dev) + 0.5, torch.randn(CV, device=dev)
+    dgam, dbet = torch.zeros(CV, device=dev), torch.zeros(CV, device=dev)
+    stats = torch.empty(2 * CV + 1, device=dev)
+    scratch = torch.empty(2, CV, device=dev)
+    xp = torch.empty(B * (TV + 1) + 2, CV, device=dev)
+    hi, lo = (torch.empty(B * (TV + 1) + 2, CV, device=dev, dtype=torch.float16) for _ in range(2))
+    xin, xin_m = torch.randn(B, TV, DV, device=dev), torch.empty(B, TV, DV, device=dev)
+    mean, var = stats[:CV], stats[CV:2 * CV]
+    vk = {
+        "bn_stats_plain": lambda: L.deer_bn_stats(p(xv), p(stats), M, CV, st()),
+        "bn_stats_len": lambda: L.deer_bn_stats_len(p(xv), p(stats), p(vlens), 0, B, TV, CV, st()),
+        "bn_relu_fwd_plain": lambda: L.deer_bn_relu_fwd(p(xv), p(mean), p(var), p(gam), p(bet), p(yv), M, CV, 1e-5,
+                                                        st()),
+        "bn_relu_fwd_len": lambda: L.deer_bn_relu_fwd_len(p(xv), p(mean), p(var), p(gam), p(bet), p(yv), p(vlens), 0, B,
+                                                          TV, CV, 1e-5, st()),
+        "bn_relu_bwd_plain": lambda: L.deer_bn_relu_bwd(p(dyv), p(xv), p(yv), p(mean), p(var), p(gam), p(dxv), p(dgam),
+                                                        p(dbet), p(scratch), M, CV, 1e-5, 1, st()),
+        "bn_relu_bwd_len": lambda: L.deer_bn_relu_bwd_len(p(dyv), p(xv), p(yv), p(mean), p(var), p(gam), p(dxv),
+                                                          p(dgam), p(dbet), p(scratch), p(vlens), 0, B, TV, CV, 1e-5, 1,
+                                                          st()),
+        "rows_pad_fwd_plain": lambda: L.deer_rows_pad_fused(p(xv), p(xp), p(hi), p(lo), B, TV, CV, 1, 1, 0, 0.0, 0, 0,
+                                                            None, st()),
+        "rows_pad_fwd_len": lambda: L.deer_rows_pad_fused_len(p(xv), p(xp), p(hi), p(lo), p(vlens), 0, B, TV, CV, 1, 1,
+                                                              0, 0.0, 0, 0, None, st()),
+        "rows_pad_bwd_plain": lambda: L.deer_rows_pad_fused(p(xp), p(dxv), None, None, B, TV, CV, 1, 1, 1, 0.0, 0, 0,
+                                                            None, st()),
+        "rows_pad_bwd_len": lambda: L.deer_rows_pad_fused_len(p(xp), p(dxv), None, None, p(vlens), 0, B, TV, CV, 1, 1,
+                                                              1, 0.0, 0, 0, None, st()),
+        "input_mask_copy_len": lambda: L.deer_rowscale_len(p(xin), p(xin_m), p(vlens), 0, B, TV, DV, st()),
+    }
+    assert L.deer_bn_stats_len(p(xv), p(stats), p(vlens), 0, B, TV, CV, st()) == 0
+    vkern_us = {}
+    for name, fn in vk.items():
+        assert fn() == 0, name
+        torch.cuda.synchronize()
+        vkern_us[name] = round(timed(fn, 200) * 1e3, 2)
+    vsum = int(vlens.long().sum())
     sum_len = int(lens.long().sum())
     rows_dense, rows_len = T * B, sum_len
     res = {
@@ -158,10 +218,15 @@ def main():
         "inference_b1024_ms": {k: round(median(v), 4) for k, v in infer_ms.items()},
         "inference_b1024_ms_all_rounds": {k: [round(x_, 4) for x_ in v] for k, v in infer_ms.items()},
         "kernel_us_b256_t300": kern_us,
+        "video_kernel_us_b256_t50_c512": vkern_us,
+        "video_bytes": {"bn_activation_pass": M * CV * 4, "input_mask_copy_read": B * TV * DV * 4,
+                        "input_mask_copy_valid_read": vsum * DV * 4},
+        "video_ragged_mean_length_b256": vsum / B,
         "pool_x_bytes_read": {"dense": rows_dense * D * 4, "len": rows_len * D * 4},
         "ragged_mean_length_b256": sum_len / B,
         "mask_pre_padded_rows_b256": rows_dense - rows_len,
         "config": {"train_batch": TRAIN_B, "inference_batch": INFER_B, "T": T, "ragged": "uniform int in [75, 300]",
+                   "video_T": TV, "video_ragged": "uniform int in [12, 50]",
                    "steps": args.steps, "rounds": args.rounds, "cuda_graphs": True},
     }
     line = json.dumps(res)

@@ -65,16 +65,22 @@ _PROTOS = {
     "deer_permute_bt_cast16_len": [P, P, P, P, I, I, I, I, I, I, P],
     "deer_scorer_bwd": [P, P, P, P, P, P, P, P, L, I, P],
     "deer_rowscale": [P, P, P, L, I, P],
+    "deer_rowscale_len": [P, P, P, I, I, I, I, P],
     "deer_im2col3": [P, P, I, I, I, P],
     "deer_col2im3": [P, P, I, I, I, P],
     "deer_rows_pad": [P, P, I, I, I, I, I, I, P],
     "deer_rows_pad_fused": [P, P, P, P, I, I, I, I, I, I, F, U, U, P, P],
+    "deer_rows_pad_fused_len": [P, P, P, P, P, I, I, I, I, I, I, I, F, U, U, P, P],
     "deer_rows_pad_colsum": [P, P, P, I, I, I, P],
     "deer_conv3_weight_pack": [P, P, I, I, I, P],
     "deer_bn_stats": [P, P, L, I, P],
     "deer_bn_update_running": [P, P, P, P, L, I, F, P],
     "deer_bn_relu_fwd": [P, P, P, P, P, P, L, I, F, P],
     "deer_bn_relu_bwd": [P, P, P, P, P, P, P, P, P, P, L, I, F, I, P],
+    "deer_bn_stats_len": [P, P, P, I, I, I, I, P],
+    "deer_bn_update_running_len": [P, P, P, P, I, F, P],
+    "deer_bn_relu_fwd_len": [P, P, P, P, P, P, P, I, I, I, I, F, P],
+    "deer_bn_relu_bwd_len": [P, P, P, P, P, P, P, P, P, P, P, I, I, I, I, F, I, P],
     "deer_mha2_fwd": [P, P, P, P, P, I, I, I, P],
     "deer_mha2_bwd": [P, P, P, P, P, P, I, I, I, P],
     "deer_lstm_fwd": [P, P, P, P, P, P, I, I, I, I, P],

@@ -99,6 +99,11 @@ __device__ __forceinline__ int seq_length(const void* lengths, int i64, int b, i
   const long long L = i64 ? static_cast<const long long*>(lengths)[b] : static_cast<const int*>(lengths)[b];
   return (int)(L < 1 ? 1 : (L > T ? T : L));
 }
+// row m of a batch-major [B*T, .] layout is (b = m / T, t = m % T): a frame of its utterance (t < L_b), not padding
+__device__ __forceinline__ bool seq_row_valid(long long m, const void* lengths, int i64, int T) {
+  const int b = (int)(m / T);
+  return (int)(m - (long long)b * T) < seq_length(lengths, i64, b, T);
+}
 
 // accurate fp32 sigmoid / tanh on the MUFU pipe (ex2 + rcp): |rel err| ~ 2 ulp
 __device__ __forceinline__ float sigmoid_f(float x) { return __fdividef(1.f, 1.f + __expf(-x)); }

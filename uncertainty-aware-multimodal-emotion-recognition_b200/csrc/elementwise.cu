@@ -299,13 +299,21 @@ __global__ void __launch_bounds__(256) lstm_mask_pre_kernel(Unit* __restrict__ p
   }
 }
 
+// kLengths: the row mask comes from per-utterance lengths (rows m = b*T + t of a [B,T,D] tensor): y = x at t < L_b and y = 0
+// at padded rows, which are not read (x * 0 would keep a NaN) -- the masked copy of a length-aware layer's input
+template <bool kLengths>
 __global__ void __launch_bounds__(256) rowscale_kernel(const float* __restrict__ x, const float* __restrict__ mask,
-                                                       float* __restrict__ y, long long M, int D) {
+                                                       float* __restrict__ y, long long M, int D, const void* lengths,
+                                                       int lengths_i64, int T) {
   DEER_PDL_ENTRY();
   const long long total = M * D;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total;
-       i += (long long)gridDim.x * blockDim.x)
-    y[i] = x[i] * mask[i / D];
+       i += (long long)gridDim.x * blockDim.x) {
+    if constexpr (kLengths)
+      y[i] = seq_row_valid(i / D, lengths, lengths_i64, T) ? x[i] : 0.f;
+    else
+      y[i] = x[i] * mask[i / D];
+  }
 }
 
 // col[(b,t), k*C + c] = x[b, t+k-1, c]
@@ -366,12 +374,17 @@ __global__ void __launch_bounds__(256) rows_pad_kernel(const float* __restrict__
 // gradient) and, optionally, its FP16 hi / lo split in the same geometry (the A operand of the split-precision forward
 // GEMM); dir 1 (backward) drops the pad rows of dx_p and applies the same mask.  Replaces dropout + rows_pad +
 // cast_split16 (three passes over the tensor) forward and rows_pad + dropout backward.
+// kLengths (per-utterance lengths): frames t >= L_b count as pad rows.  dir 0 writes zeros for them (their source rows are
+// not read), so the convolution sees each clip zero-padded at both ends; dir 1 writes dx = 0 for them -- dx_p row L_b holds
+// the tap dy[L_b - 1] W, which would otherwise leak into the padded rows' gradient.
+template <bool kLengths>
 __global__ void __launch_bounds__(256) rows_pad_fused_kernel(const float* __restrict__ src, float* __restrict__ dst,
                                                              uint16_t* __restrict__ hi, uint16_t* __restrict__ lo, int B,
                                                              int T, int C4, int lead, int dir, long long pad_rows_total,
                                                              float p, float scale, unsigned long long seed,
                                                              unsigned long long offset,
-                                                             const unsigned long long* __restrict__ step_ptr) {
+                                                             const unsigned long long* __restrict__ step_ptr,
+                                                             const void* lengths, int lengths_i64) {
   DEER_PDL_ENTRY();
   const unsigned long long st = step_ptr ? *step_ptr : 0ull;
   const uint32_t thr = (uint32_t)fminf(p * 4294967296.f, 4294967040.f);
@@ -391,10 +404,10 @@ __global__ void __launch_bounds__(256) rows_pad_fused_kernel(const float* __rest
       if (q >= 0) {
         const long long b = q / (T + 1);
         const int t = (int)(q % (T + 1));
-        if (b < B && t < T) ci = (b * T + t) * C4 + c;
+        if (b < B && t < T && (!kLengths || t < seq_length(lengths, lengths_i64, (int)b, T))) ci = (b * T + t) * C4 + c;
       }
     } else {
-      ci = i;
+      ci = (!kLengths || seq_row_valid(r, lengths, lengths_i64, T)) ? i : -1;
     }
     float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
     if (ci >= 0) {
@@ -808,7 +821,14 @@ int deer_lstm_mask_pre(void* pre, int pre_fp16, const void* lengths, int lengths
 
 int deer_rowscale(const float* x, const float* mask, float* y, long long M, int D, void* stream) {
   DEER_CHECK_ARG(x && mask && y && M > 0 && D > 0, "rowscale: bad args");
-  DEER_LAUNCH(rowscale_kernel, grid_for(M * D), 256, 0, stream, x, mask, y, M, D);
+  DEER_LAUNCH(rowscale_kernel<false>, grid_for(M * D), 256, 0, stream, x, mask, y, M, D, nullptr, 0, 1);
+  return DEER_OK;
+}
+
+int deer_rowscale_len(const float* x, float* y, const void* lengths, int lengths_i64, int B, int T, int D, void* stream) {
+  DEER_CHECK_ARG(x && y && lengths && B > 0 && T > 0 && D > 0, "rowscale_len: bad args");
+  const long long M = (long long)B * T;
+  DEER_LAUNCH(rowscale_kernel<true>, grid_for(M * D), 256, 0, stream, x, nullptr, y, M, D, lengths, lengths_i64, T);
   return DEER_OK;
 }
 
@@ -828,9 +848,9 @@ int deer_rows_pad(const float* src, float* dst, int B, int T, int C, int lead, i
   return DEER_OK;
 }
 
-int deer_rows_pad_fused(const float* src, float* dst, void* hi, void* lo, int B, int T, int C, int lead, int tail, int dir,
-                        float drop_p, unsigned long long seed, unsigned long long offset, const unsigned long long* step_ptr,
-                        void* stream) {
+static int rows_pad_fused(const float* src, float* dst, void* hi, void* lo, int B, int T, int C, int lead, int tail,
+                          int dir, float drop_p, unsigned long long seed, unsigned long long offset,
+                          const unsigned long long* step_ptr, const void* lengths, int lengths_i64, void* stream) {
   DEER_CHECK_ARG(src && dst && B > 0 && T > 0 && C > 0 && (C & 3) == 0 && lead >= 0 && tail >= 0 && (dir == 0 || dir == 1) &&
                      drop_p >= 0.f && drop_p < 1.f && ((hi == nullptr) == (lo == nullptr)) && (dir == 0 || hi == nullptr),
                  "rows_pad_fused: bad args");
@@ -839,10 +859,24 @@ int deer_rows_pad_fused(const float* src, float* dst, void* hi, void* lo, int B,
                  "rows_pad_fused: alignment");
   const long long pad_rows = (long long)lead + (long long)B * (T + 1) + tail;
   const long long n4 = (dir == 0 ? pad_rows : (long long)B * T) * (C / 4);
-  DEER_LAUNCH(rows_pad_fused_kernel, grid_for(n4), 256, 0, stream, src, dst, reinterpret_cast<uint16_t*>(hi),
-              reinterpret_cast<uint16_t*>(lo), B, T, C / 4, lead, dir, pad_rows, drop_p, 1.f / (1.f - drop_p), seed, offset,
-              step_ptr);
+  DEER_LAUNCH(lengths ? rows_pad_fused_kernel<true> : rows_pad_fused_kernel<false>, grid_for(n4), 256, 0, stream, src,
+              dst, reinterpret_cast<uint16_t*>(hi), reinterpret_cast<uint16_t*>(lo), B, T, C / 4, lead, dir, pad_rows,
+              drop_p, 1.f / (1.f - drop_p), seed, offset, step_ptr, lengths, lengths_i64);
   return DEER_OK;
+}
+
+int deer_rows_pad_fused(const float* src, float* dst, void* hi, void* lo, int B, int T, int C, int lead, int tail, int dir,
+                        float drop_p, unsigned long long seed, unsigned long long offset, const unsigned long long* step_ptr,
+                        void* stream) {
+  return rows_pad_fused(src, dst, hi, lo, B, T, C, lead, tail, dir, drop_p, seed, offset, step_ptr, nullptr, 0, stream);
+}
+
+int deer_rows_pad_fused_len(const float* src, float* dst, void* hi, void* lo, const void* lengths, int lengths_i64, int B,
+                            int T, int C, int lead, int tail, int dir, float drop_p, unsigned long long seed,
+                            unsigned long long offset, const unsigned long long* step_ptr, void* stream) {
+  DEER_CHECK_ARG(lengths, "rows_pad_fused_len: bad args");
+  return rows_pad_fused(src, dst, hi, lo, B, T, C, lead, tail, dir, drop_p, seed, offset, step_ptr, lengths, lengths_i64,
+                        stream);
 }
 
 int deer_rows_pad_colsum(const float* src, float* dst, float* colsum, int B, int T, int C, void* stream) {

@@ -142,16 +142,31 @@ class EnhancedVideoEncoder(nn.Module):
         self.temporal_attention = nn.Sequential(nn.Linear(d, d // 2), nn.Tanh(), nn.Linear(d // 2, 1), nn.Softmax(dim=1))
         self.output_projection = nn.Sequential(nn.Linear(d, d), nn.ReLU(), nn.Dropout(self.dropout), nn.LayerNorm(d))
 
-    def _bn_relu(self, x, bn: nn.BatchNorm1d):
+    def _bn_relu(self, x, bn: nn.BatchNorm1d, lengths=None):
         return ops.batchnorm_relu(x, bn.weight, bn.bias, bn.running_mean, bn.running_var, bn.num_batches_tracked,
-                                  self.training, bn.momentum, bn.eps)
+                                  self.training, bn.momentum, bn.eps, lengths=lengths)
 
-    def forward(self, video_input: torch.Tensor) -> torch.Tensor:
+    def forward(self, video_input: torch.Tensor, lengths: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """video_input [B,T,frame_feature_dim] per-frame features.  `lengths` [B] (int32 / int64, CUDA or CPU; None: every
+        clip has all T frames): sample b is the clip video_input[b, :L_b].  Each Conv1d sees the clip zero-padded at its
+        own ends, BatchNorm (training) takes its statistics over the valid frames of the batch only (nn.BatchNorm1d on
+        them packed into one batch, running statistics included), BN+ReLU is 0 at padded frames and the attention
+        softmax covers t < L_b -- so in eval a clip's encoding equals that of the clip alone, and the content of the
+        padded frames (zeros, noise, NaN) changes no output or gradient; the input gradient is 0 there.  A clip with
+        L_b = 1 in a batch with T > 1 still goes through the convolutions and BatchNorm (on its one frame); the
+        reference's one-frame shortcut (no convolution, no BatchNorm) applies only when T itself is 1, and lengths then
+        have no effect.  CUDA lengths are clamped to [1, T] on the device; CPU lengths outside that range raise."""
         if video_input.dim() == 2:
             video_input = video_input.unsqueeze(1)
         if video_input.dim() != 3:
             raise NotImplementedError("deer_b200: raw frames / the 2-D CNN backbone are outside the CUDA hot path; pass "
                                       "per-frame features [B,F,frame_feature_dim]")
+        lengths = ops.sequence_lengths(lengths, video_input.shape[0], video_input.shape[1], video_input.device)
+        if lengths is not None and video_input.shape[1] == 1:
+            lengths = None
+        if lengths is not None:
+            # padded rows of the input become zero rows (never read): spatial_projection's dW = dz^T x takes no 0 * NaN
+            video_input = ops.mask_padding(video_input, lengths)
         sp, cnn = self.spatial_projection, self.temporal_cnn
         p = ops.linear(video_input, sp[0].weight, sp[0].bias, "relu")
         # the autograd node that runs LAST in this encoder's backward: the data-parallel trainer hangs its early
@@ -159,11 +174,11 @@ class EnhancedVideoEncoder(nn.Module):
         self.__dict__["_first_bwd_node"] = p.grad_fn
         if video_input.shape[1] > 1:
             # the two nn.Dropout layers in front of the convolutions ride on the convolutions' padding passes
-            h = ops.conv1d_k3(p, cnn[0].weight, cnn[0].bias, self.dropout, self.training)
-            h = self._bn_relu(h, cnn[1])
-            h = ops.conv1d_k3(h, cnn[4].weight, cnn[4].bias, self.dropout, self.training)
-            h = self._bn_relu(h, cnn[5])
-            pooled, _ = _scorer_and_pool(h, self.temporal_attention)
+            h = ops.conv1d_k3(p, cnn[0].weight, cnn[0].bias, self.dropout, self.training, lengths=lengths)
+            h = self._bn_relu(h, cnn[1], lengths)
+            h = ops.conv1d_k3(h, cnn[4].weight, cnn[4].bias, self.dropout, self.training, lengths=lengths)
+            h = self._bn_relu(h, cnn[5], lengths)
+            pooled, _ = _scorer_and_pool(h, self.temporal_attention, lengths=lengths)
         else:
             pooled = ops.dropout(p, self.dropout, self.training)[:, 0]
         op = self.output_projection

@@ -1036,6 +1036,35 @@ def rowscale(x, mask):
     return _RowScale.apply(x, mask)
 
 
+def _mask_padding(x, lengths):
+    B, T, D = x.shape
+    y = torch.empty_like(x)
+    call("deer_rowscale_len", ptr(x), ptr(y), lengths.data_ptr(), _len_i64(lengths), B, T, D)
+    return y
+
+
+class _MaskPadding(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, lengths):
+        ctx.lengths = lengths
+        return _mask_padding(x, lengths)
+
+    @staticmethod
+    def backward(ctx, dy):
+        return _mask_padding(dy.contiguous(), ctx.lengths), None
+
+
+def mask_padding(x, lengths):
+    """x [B,T,D] with the padded frames t >= L_b (lengths: see sequence_lengths) replaced by zero rows, which are never
+    read (NaN padding stays out).  An autograd node only when x needs a gradient; its backward is the same masked copy,
+    so the input gradient is exactly 0 at padded frames."""
+    x = _req(x, "x").contiguous()
+    lengths = sequence_lengths(lengths, x.shape[0], x.shape[1], x.device)
+    if x.requires_grad and torch.is_grad_enabled():
+        return _MaskPadding.apply(x, lengths)
+    return _mask_padding(x, lengths)
+
+
 def linguistic_features(input_ids: torch.Tensor, attention_mask: torch.Tensor, max_length: int = 128) -> torch.Tensor:
     """EnhancedTextEncoder.extract_linguistic_features (encoders.py:648-699) as one integer kernel: [B,T] int64 token
     ids + mask -> [B,10] fp32 (no gradient path, as in the reference)."""
@@ -1516,13 +1545,17 @@ def bilstm_layer(x_tm, wif, whf, bif, bhf, wir, whr, bir, bhr, input_dropout: fl
 
 # ----------------------------------------------------------------------------------------------- Conv1d(k=3) + BN
 class _Conv1dK3(torch.autograd.Function):
-    """nn.Conv1d(Cin,Cout,3,padding=1) on channels-last x [B,T,Cin] -> [B,T,Cout]; w [Cout,Cin,3]."""
+    """nn.Conv1d(Cin,Cout,3,padding=1) on channels-last x [B,T,Cin] -> [B,T,Cout]; w [Cout,Cin,3].  lengths (device [B]):
+    each clip x[b, :L_b] is convolved alone -- x is masked to zero rows at t >= L_b before the im2col, and dx after the
+    col2im (0 at padded frames)."""
 
     @staticmethod
-    def forward(ctx, x, w, b):
+    def forward(ctx, x, w, b, lengths=None):
         x = _req(x, "x").contiguous()
         B, T, Cin = x.shape
         Cout = w.shape[0]
+        if lengths is not None:
+            x = _mask_padding(x, lengths)
         col = torch.empty((B * T, 3 * Cin), device=x.device, dtype=torch.float32)
         call("deer_im2col3", ptr(x), ptr(col), B, T, Cin)
         wk = torch.empty((Cout, 3 * Cin), device=x.device, dtype=torch.float32)
@@ -1536,6 +1569,7 @@ class _Conv1dK3(torch.autograd.Function):
         ctx.save_for_backward(col, wk)
         ctx.dims = (B, T, Cin, Cout)
         ctx.params = (w, b)
+        ctx.lengths = lengths
         return y
 
     @staticmethod
@@ -1551,6 +1585,8 @@ class _Conv1dK3(torch.autograd.Function):
                  engine=_state["exact_engine"] if (_state["conv_exact"] & 2) else None)
             dx = torch.empty((B, T, Cin), device=dy.device, dtype=torch.float32)
             call("deer_col2im3", ptr(dcol), ptr(dx), B, T, Cin)
+            if ctx.lengths is not None:
+                dx = _mask_padding(dx, ctx.lengths)
         dwk = zeros_scratch(tuple(wk.shape), dy.device)
         gemm(dy, Cout, 1, col, 3 * Cin, 0, dwk, 3 * Cin, Cout, 3 * Cin, M, beta=1.0,
              engine=_state["exact_engine"] if (_state["conv_exact"] & 2) else None)
@@ -1558,7 +1594,7 @@ class _Conv1dK3(torch.autograd.Function):
         call("deer_conv3_weight_pack", ptr(dwk), ptr(dw), Cout, Cin, 1)
         db, db_direct = _acc(ctx.params[1])
         call("deer_bias_act_bwd", ptr(dy), Cout, None, 0, None, 0, ptr(db), M, Cout, 0)
-        return dx, None if dw_direct else dw, None if db_direct else db
+        return dx, None if dw_direct else dw, None if db_direct else db, None
 
 
 class _Conv1dK3Window(torch.autograd.Function):
@@ -1570,9 +1606,11 @@ class _Conv1dK3Window(torch.autograd.Function):
     Rows centred on a pad row are garbage in y_big and are dropped by the un-padding copy; dy_big has zeros there."""
 
     @staticmethod
-    def forward(ctx, x, w, b, drop=None):
+    def forward(ctx, x, w, b, drop=None, lengths=None):
         """drop = (p, seed, offset, step tensor or None): the nn.Dropout in front of the convolution (encoders.py:453-454)
-        folded into the padding pass (forward) and the un-padding pass (backward): same Philox stream as ops.dropout."""
+        folded into the padding pass (forward) and the un-padding pass (backward): same Philox stream as ops.dropout.
+        lengths (device [B]): frames t >= L_b are pad rows of xp as well (zeros, not read), and the un-padding pass of
+        the backward writes dx = 0 there."""
         x = _req(x, "x").contiguous()
         B, T, Cin = x.shape
         Cout = w.shape[0]
@@ -1586,8 +1624,7 @@ class _Conv1dK3Window(torch.autograd.Function):
             xh = torch.empty((Mp + 2, Cin), device=dev, dtype=torch.float16)
             xl = torch.empty((Mp + 2, Cin), device=dev, dtype=torch.float16)
         # one pass: dropout, zero pad rows, fp32 copy (weight gradient) and the split-precision A operand
-        call("deer_rows_pad_fused", ptr(x), ptr(xp), None if xh is None else xh.data_ptr(),
-             None if xl is None else xl.data_ptr(), B, T, Cin, 1, 1, 0, float(dp), int(dseed), int(doff), ptr(dstep))
+        _rows_pad_fused(x, xp, xh, xl, lengths, B, T, Cin, 0, float(dp), int(dseed), int(doff), dstep)
         wk = torch.empty((Cout, 3 * Cin), device=dev, dtype=torch.float32)
         call("deer_conv3_weight_pack", ptr(w.contiguous()), ptr(wk), Cout, Cin, 0)
         y_big = torch.empty((Mp, Cout), device=dev, dtype=torch.float32)
@@ -1602,6 +1639,7 @@ class _Conv1dK3Window(torch.autograd.Function):
         ctx.dims = (B, T, Cin, Cout)
         ctx.params = (w, b)
         ctx.drop = (float(dp), int(dseed), int(doff), dstep)
+        ctx.lengths = lengths
         return y
 
     @staticmethod
@@ -1629,7 +1667,7 @@ class _Conv1dK3Window(torch.autograd.Function):
                 gemm(dy_big, Cout, 0, wk, 3 * Cin, 0, dx_p, Cin, Mp, 3 * Cin, Cout, beta=1.0)   # ldc = Cin < N: overlapped
             dx = torch.empty((B, T, Cin), device=dev, dtype=torch.float32)
             dp, dseed, doff, dstep = ctx.drop
-            call("deer_rows_pad_fused", ptr(dx_p), ptr(dx), None, None, B, T, Cin, 1, 1, 1, dp, dseed, doff, ptr(dstep))
+            _rows_pad_fused(dx_p, dx, None, None, ctx.lengths, B, T, Cin, 1, dp, dseed, doff, dstep)
         dwk = zeros_scratch(tuple(wk.shape), dev)
         if bf:
             gemm_h16(dyb, Cout, 1, xpb, Cin, 0, dwk, 3 * Cin, Cout, 3 * Cin, Mp, a_bf16=True, b_bf16=True, beta=1.0)
@@ -1637,7 +1675,19 @@ class _Conv1dK3Window(torch.autograd.Function):
             gemm(dy_big, Cout, 1, xp, Cin, 0, dwk, 3 * Cin, Cout, 3 * Cin, Mp, beta=1.0)         # ldb = Cin < N = 3 Cin
         dw, dw_direct = _acc(ctx.params[0])
         call("deer_conv3_weight_pack", ptr(dwk), ptr(dw), Cout, Cin, 1)
-        return dx, None if dw_direct else dw, None if db_direct else db, None
+        return dx, None if dw_direct else dw, None if db_direct else db, None, None
+
+
+def _rows_pad_fused(src, dst, hi, lo, lengths, B, T, C, direction, dp, dseed, doff, dstep):
+    """The sliding-window convolution's padding (direction 0) / un-padding (1) pass, lead = tail = 1 row; with lengths
+    the frames t >= L_b are pad rows too."""
+    hp = None if hi is None else hi.data_ptr()
+    lp = None if lo is None else lo.data_ptr()
+    if lengths is not None:
+        call("deer_rows_pad_fused_len", ptr(src), ptr(dst), hp, lp, lengths.data_ptr(), _len_i64(lengths), B, T, C, 1, 1,
+             direction, dp, dseed, doff, ptr(dstep))
+    else:
+        call("deer_rows_pad_fused", ptr(src), ptr(dst), hp, lp, B, T, C, 1, 1, direction, dp, dseed, doff, ptr(dstep))
 
 
 def set_conv_window(on: bool):
@@ -1645,13 +1695,17 @@ def set_conv_window(on: bool):
     _state["conv_window"] = bool(on)
 
 
-def conv1d_k3(x, w, b, dropout_p: float = 0.0, training: bool = False):
+def conv1d_k3(x, w, b, dropout_p: float = 0.0, training: bool = False, lengths=None):
     """Conv1d(k=3, padding=1) of dropout(x) (dropout_p > 0 and training: the nn.Dropout in front of the convolution,
     encoders.py:453-454).  Large batches on the TMA engine use the sliding-window path (no im2col matrix; the dropout
     rides on its padding / un-padding passes); small ones (the CTA-pair kernel needs > 256 rows), forced engines and odd
-    channel counts keep the im2col + GEMM path behind a separate dropout node.  Both draw the same masks."""
+    channel counts keep the im2col + GEMM path behind a separate dropout node.  Both draw the same masks.
+    `lengths` [B] (see sequence_lengths): sample b is the clip x[b, :L_b], convolved with zero padding at both of ITS
+    ends (the tap at t = L_b reads 0); the output rows t >= L_b are finite but meaningless, and the input gradient is
+    exactly 0 there."""
     B, T, Cin = x.shape
     Cout = w.shape[0]
+    lengths = sequence_lengths(lengths, B, T, x.device)
     dropping = training and dropout_p > 0.0
     if (_state.get("conv_window", True) and not _state["conv_exact"] and _state["engine"] == ENGINE_AUTO and
             B * (T + 1) > 256 and Cin % 4 == 0 and
@@ -1663,10 +1717,10 @@ def conv1d_k3(x, w, b, dropout_p: float = 0.0, training: bool = False):
             drop = (float(dropout_p), _dropout_seed(), off, _dropout_state["step"])
         elif dropping:
             x = dropout(x, dropout_p, training)
-        return _Conv1dK3Window.apply(x, w, b, drop)
+        return _Conv1dK3Window.apply(x, w, b, drop, lengths)
     if dropping:
         x = dropout(x, dropout_p, training)
-    return _Conv1dK3.apply(x, w, b)
+    return _Conv1dK3.apply(x, w, b, lengths)
 
 
 def set_conv_dropout_fused(on: bool):
@@ -1676,26 +1730,44 @@ def set_conv_dropout_fused(on: bool):
 
 
 class _BNReLU(torch.autograd.Function):
-    """nn.BatchNorm1d (channels-last rows) followed by ReLU."""
+    """nn.BatchNorm1d (channels-last rows) followed by ReLU.  lengths (device [B], x [B,T,C]): the rows are the valid
+    frames t < L_b only -- nn.BatchNorm1d on those packed into one [N, C] batch, N = sum_b L_b counted on the device
+    (stats [2C+1]: mean, biased var, N); y = 0 and dx = 0 at padded rows."""
 
     @staticmethod
-    def forward(ctx, x, g, b, running_mean, running_var, nbt, training, momentum, eps):
+    def forward(ctx, x, g, b, running_mean, running_var, nbt, training, momentum, eps, lengths=None):
         x = _req(x, "x").contiguous()
         C = x.shape[-1]
         M = x.numel() // C
         y = torch.empty_like(x)
+        nbt_p = None if nbt is None else nbt.data_ptr()
+        if lengths is not None:
+            B, T = x.shape[0], x.shape[1]
+            lp, li = lengths.data_ptr(), _len_i64(lengths)
         if training:
-            stats = torch.empty((2, C), device=x.device, dtype=torch.float32)
-            call("deer_bn_stats", ptr(x), ptr(stats), M, C)
-            call("deer_bn_update_running", ptr(stats), ptr(running_mean), ptr(running_var),
-                 None if nbt is None else nbt.data_ptr(), M, C, float(momentum))
-            mean, var = stats[0], stats[1]
+            if lengths is not None:
+                stats = torch.empty(2 * C + 1, device=x.device, dtype=torch.float32)
+                call("deer_bn_stats_len", ptr(x), ptr(stats), lp, li, B, T, C)
+                call("deer_bn_update_running_len", ptr(stats), ptr(running_mean), ptr(running_var), nbt_p, C,
+                     float(momentum))
+                mean, var = stats[:C], stats[C:2 * C]     # views: the backward reads N at mean[2C]
+            else:
+                stats = torch.empty((2, C), device=x.device, dtype=torch.float32)
+                call("deer_bn_stats", ptr(x), ptr(stats), M, C)
+                call("deer_bn_update_running", ptr(stats), ptr(running_mean), ptr(running_var), nbt_p, M, C,
+                     float(momentum))
+                mean, var = stats[0], stats[1]
         else:
             mean, var = running_mean, running_var
-        call("deer_bn_relu_fwd", ptr(x), ptr(mean), ptr(var), ptr(g), ptr(b), ptr(y), M, C, float(eps))
+        if lengths is not None:
+            call("deer_bn_relu_fwd_len", ptr(x), ptr(mean), ptr(var), ptr(g), ptr(b), ptr(y), lp, li, B, T, C,
+                 float(eps))
+        else:
+            call("deer_bn_relu_fwd", ptr(x), ptr(mean), ptr(var), ptr(g), ptr(b), ptr(y), M, C, float(eps))
         ctx.save_for_backward(x, y, mean.clone() if not training else mean, var.clone() if not training else var, g)
         ctx.cfg = (M, C, float(eps), bool(training))
         ctx.params = (g, b)
+        ctx.lengths = lengths
         return y
 
     @staticmethod
@@ -1707,13 +1779,25 @@ class _BNReLU(torch.autograd.Function):
         dg, dg_direct = _acc(ctx.params[0])
         db, db_direct = _acc(ctx.params[1])
         scratch = torch.empty((2, C), device=x.device, dtype=torch.float32)
-        call("deer_bn_relu_bwd", ptr(dy), ptr(x), ptr(y), ptr(mean), ptr(var), ptr(g), ptr(dx), ptr(dg), ptr(db),
-             ptr(scratch), M, C, eps, int(training))
-        return dx, None if dg_direct else dg, None if db_direct else db, None, None, None, None, None, None
+        lengths = ctx.lengths
+        if lengths is not None:
+            call("deer_bn_relu_bwd_len", ptr(dy), ptr(x), ptr(y), ptr(mean), ptr(var), ptr(g), ptr(dx), ptr(dg),
+                 ptr(db), ptr(scratch), lengths.data_ptr(), _len_i64(lengths), x.shape[0], x.shape[1], C, eps,
+                 int(training))
+        else:
+            call("deer_bn_relu_bwd", ptr(dy), ptr(x), ptr(y), ptr(mean), ptr(var), ptr(g), ptr(dx), ptr(dg), ptr(db),
+                 ptr(scratch), M, C, eps, int(training))
+        return dx, None if dg_direct else dg, None if db_direct else db, None, None, None, None, None, None, None
 
 
-def batchnorm_relu(x, g, b, running_mean, running_var, nbt, training, momentum=0.1, eps=1e-5):
-    return _BNReLU.apply(x, g, b, running_mean, running_var, nbt, training, momentum, eps)
+def batchnorm_relu(x, g, b, running_mean, running_var, nbt, training, momentum=0.1, eps=1e-5, lengths=None):
+    """`lengths` [B] (see sequence_lengths) with x [B,T,C]: the statistics, the output and the gradients cover the frames
+    t < L_b only; padded rows of y and dx are exactly 0 and their content in x does not matter."""
+    if lengths is not None:
+        if x.dim() != 3:
+            raise _lib.DeerError(f"deer_b200: batchnorm_relu with lengths needs x [B,T,C], got {tuple(x.shape)}")
+        lengths = sequence_lengths(lengths, x.shape[0], x.shape[1], x.device)
+    return _BNReLU.apply(x, g, b, running_mean, running_var, nbt, training, momentum, eps, lengths)
 
 
 # ----------------------------------------------------------------------------------------------- 2-token MHA core

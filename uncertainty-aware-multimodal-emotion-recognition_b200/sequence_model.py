@@ -33,9 +33,11 @@ class SequenceDEERModel(nn.Module):
 
     def forward(self, audio, video=None, text=None, attention_mask: Optional[torch.Tensor] = None,
                 linguistic_features: Optional[torch.Tensor] = None,
-                audio_lengths: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
+                audio_lengths: Optional[torch.Tensor] = None,
+                video_lengths: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
         """`audio_lengths` [B] (int32 / int64; also read from the batch dict key "audio_lengths"): frames of each audio
-        utterance, see EnhancedAudioEncoder.forward.  None: every sample has all T frames."""
+        utterance, see EnhancedAudioEncoder.forward.  `video_lengths` [B] (batch key "video_lengths"): frames of each
+        video clip, see EnhancedVideoEncoder.forward.  None: every sample has all T frames."""
         if isinstance(audio, dict):
             d = audio
             audio = d.get("audio", d.get("audio_features"))
@@ -44,6 +46,7 @@ class SequenceDEERModel(nn.Module):
             attention_mask = d.get("attention_mask", attention_mask)
             linguistic_features = d.get("linguistic_features", linguistic_features)
             audio_lengths = d.get("audio_lengths", audio_lengths)
+            video_lengths = d.get("video_lengths", video_lengths)
         ops.begin_step()
         # training: up to 512 samples the recurrence is ONE wave of clusters; beyond that the second wave of the
         # (gate / cell storing) kernels competes with the side work for SMs.  Inference forwards (no stores for BPTT,
@@ -72,7 +75,7 @@ class SequenceDEERModel(nn.Module):
             # program order video -> text (whatever the streams): the video encoder's first node keeps the lowest sequence
             # number behind the audio block, so autograd runs it LAST in backward -- the trainer's early gradient exchange
             # hangs its "everything behind the audio block is complete" hook on it
-            v = ops.mark_tensor(self.video_encoder(ops.mark_tensor(video, "video_in")), "video_out")
+            v = ops.mark_tensor(self.video_encoder(ops.mark_tensor(video, "video_in"), video_lengths), "video_out")
             if tside is None:
                 t = ops.mark_tensor(self.text_encoder(ops.mark_tensor(text, "text_in"), attention_mask,
                                                       linguistic_features), "text_out")
@@ -87,7 +90,7 @@ class SequenceDEERModel(nn.Module):
             ops.mark("joined")
         else:
             a = self.audio_encoder(audio, audio_lengths)
-            v = self.video_encoder(video)
+            v = self.video_encoder(video, video_lengths)
             t = self.text_encoder(text, attention_mask, linguistic_features)
         if chain.enabled() and a.is_cuda and chain.supported(self.fusion, self.deer, a, v, t):
             # fusion + NIG head as ONE persistent-kernel launch (and one in backward): csrc/chain.cu

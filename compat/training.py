@@ -131,7 +131,7 @@ class DEERTrainer:
         self.model.eval()
         total, n = torch.zeros((), device=self.device), 0
         for b in DevicePrefetcher((x for loader in val_loaders.values() for x in loader), self.device):
-            total += self.model.compute_loss(self.model(b), b["targets"])["total_loss"]
+            total += self.model.compute_loss(self.model(b), b["targets"], b.get("target_mask"))["total_loss"]
             n += 1
         self.model.train()
         return {"val_loss": float(total) / max(n, 1), "val_ccc": m["mean_ccc"], **m}

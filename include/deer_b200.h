@@ -356,6 +356,25 @@ int deer_nig_loss_finish(const float* evidence, const float* gamma, const float*
                          const float* task_weights /* [D] or NULL */, float reg_w, float kl_w, float ece_w,
                          float cross_w, float eps, long long B_local, long long B_global, int D, int from_evidence,
                          float grad_scale, float* losses, float* d_out /* [B,D,4] */, void* stream);
+/*      partially labelled batches: target_mask [B,D] (bool / uint8 bytes, device memory), nonzero = labelled.  The same
+ *      kernels as the two entries above; per dimension d the means, the ECE bins (bin weight n_k / N_d) and the mean
+ *      uncertainty cover only the N_d labelled elements, the cross-dimension term averages over the pairs of dimensions
+ *      that both have N > 0 (0 with fewer than two), a dimension with N_d = 0 gets five 0 loss entries, and the gradient
+ *      is exactly 0 at every unlabelled element.  Target values at unlabelled elements are never used (NaN / Inf there
+ *      change nothing); nig_out is still written for every element.  Phase 1 accumulates N_d into stats[d*NSTAT + 35],
+ *      an fp32 sum like the ECE bin counts: exact up to 2^24 labelled elements per dimension (the all-reduced total for
+ *      a data-parallel caller).  Phase 2 takes N_d from there, so there is no B_global; block 0 writes N_d to
+ *      counts[D] when counts is not NULL (it requires losses).  losses[5D+2] has the layout above. */
+int deer_nig_loss_stats_mask(const float* evidence, const float* gamma, const float* nu, const float* alpha,
+                             const float* beta, const float* targets, const void* target_mask, const float* bin_edges,
+                             float* stats, float* nig_out /* [7,B,D] or NULL */, long long B, int D, int from_evidence,
+                             float eps, void* stream);
+int deer_nig_loss_finish_mask(const float* evidence, const float* gamma, const float* nu, const float* alpha,
+                              const float* beta, const float* targets, const void* target_mask,
+                              const float* bin_edges, const float* stats, const float* task_weights /* [D] or NULL */,
+                              float reg_w, float kl_w, float ece_w, float cross_w, float eps, long long B_local, int D,
+                              int from_evidence, float grad_scale, float* losses, float* d_out /* [B,D,4] or NULL */,
+                              float* counts /* [D] or NULL */, void* stream);
 /*      Amini-style variant, deer.py:111-195 (L3): stats-free single pass + mean; losses[5] */
 int deer_amini_loss(const float* mu, const float* nu, const float* alpha, const float* beta, const float* targets,
                     float evidence_w, float kl_w, long long N, float* losses, float* dparams /* [4,N] or NULL */,

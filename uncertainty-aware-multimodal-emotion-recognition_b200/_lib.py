@@ -99,6 +99,8 @@ _PROTOS = {
     "deer_nig_head_bwd": [P, P, P, P, P, P, P, P, P, L, P],
     "deer_nig_loss_stats": [P, P, P, P, P, P, P, P, P, L, I, I, F, P],
     "deer_nig_loss_finish": [P, P, P, P, P, P, P, P, P, F, F, F, F, F, L, L, I, I, F, P, P, P],
+    "deer_nig_loss_stats_mask": [P, P, P, P, P, P, P, P, P, P, L, I, I, F, P],
+    "deer_nig_loss_finish_mask": [P, P, P, P, P, P, P, P, P, P, F, F, F, F, F, L, I, I, F, P, P, P, P],
     "deer_amini_loss": [P, P, P, P, P, F, F, L, P, P, P, P],
     "deer_sumsq": [P, L, P, P],
     "deer_fill_zero": [P, L, P, L, P],

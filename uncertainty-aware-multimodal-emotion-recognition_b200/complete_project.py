@@ -262,8 +262,12 @@ class CompleteDEERModel(nn.Module):
         out["fused_features"] = fused
         return out
 
-    def compute_loss(self, predictions: Dict[str, torch.Tensor], targets: torch.Tensor) -> Dict[str, torch.Tensor]:
-        return self.loss_fn(predictions, targets)
+    def compute_loss(self, predictions: Dict[str, torch.Tensor], targets: torch.Tensor,
+                     target_mask: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
+        """`target_mask` (targets' shape, bool / uint8, nonzero = labelled): partially labelled batch, see losses."""
+        if target_mask is None:
+            return self.loss_fn(predictions, targets)
+        return self.loss_fn(predictions, targets, target_mask=target_mask)
 
     def get_predictions_and_uncertainties(self, outputs: Dict[str, torch.Tensor]) -> Tuple[torch.Tensor, torch.Tensor]:
         return outputs["mu_all"], outputs.get("calibrated_uncertainty", outputs["uncertainty_all"])

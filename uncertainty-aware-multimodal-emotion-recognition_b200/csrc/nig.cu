@@ -14,11 +14,19 @@
 //   phase 2 (deer_nig_loss_finish) turns the statistics into the loss scalars (block 0) and streams the
 //           analytic gradient: reads 16+4 B, writes 16 B per element.
 // A data-parallel caller all-reduces `stats` between the phases (B_global = global batch).
+//
+// Partially labelled batches (kMask, deer_nig_loss_*_mask): one more byte per element, target_mask[e] != 0 = labelled.
+// Phase 1 substitutes gamma for the target of an unlabelled element (err = 0: every intermediate stays finite whatever
+// the target holds) and SELECTS its statistic contributions and ECE bin update to nothing (0 * NaN would be NaN); it
+// counts the labelled elements of each dimension into statistic 35.  Phase 2 divides by that per-dimension N_d instead
+// of B_global, forms the cross-dimension term over the dimensions with N_d > 0 and stores a zero gradient at
+// unlabelled elements.  The kMask = false instantiations are the kernels of the plain entries, unchanged.
 #include "common.cuh"
 
 namespace deer {
 
-constexpr int NSTAT = DEER_LOSS_NSTAT;  // 0 nll,1 reg,2 kl_alpha,3 kl_beta,4 sum u, 5..14 cnt, 15..24 conf, 25..34 err
+constexpr int NSTAT = DEER_LOSS_NSTAT;  // 0 nll,1 reg,2 kl_alpha,3 kl_beta,4 sum u, 5..14 cnt, 15..24 conf, 25..34 err,
+                                        // 35 labelled count (mask entries only)
 constexpr int LOSS_THREADS = 192;       // multiple of every supported D (1,2,3,4,6,8)
 constexpr int LOSS_MIN_BLOCKS = 5;      // 64 registers: two P2 pairs in flight per thread without spills
 constexpr int LOSS_MIN_BLOCKS_PIPE = 4; // 80 registers: + the next trip's operands (software-pipelined loads)
@@ -168,7 +176,8 @@ __device__ __forceinline__ V digamma_ge1_fast(V x) {
 // each thread keeps LOSS_UNROLL independent 128-bit loads in flight (the kernels are otherwise latency-bound)
 struct RawNig {
   float4 v;  // evidence, or (gamma, nu, alpha, beta)
-  float y;
+  float y;   // target (gamma when unlabelled)
+  bool lab;  // labelled (always true without a mask)
 };
 // L2 residency control.  The loss is two passes over the same 20 B per element; when the operands fit in L2 the first
 // pass loads them with an evict_last policy so that the second pass (streaming loads, which demote the lines again) is
@@ -190,12 +199,18 @@ __device__ __forceinline__ float ld_keep_f(const float* p, unsigned long long po
   asm volatile("ld.global.L2::cache_hint.f32 %0, [%1], %2;" : "=f"(v) : "l"(p), "l"(pol));
   return v;
 }
-template <bool KEEP, bool from_evidence>
+__device__ __forceinline__ unsigned ld_keep_u8(const unsigned char* p, unsigned long long pol) {
+  unsigned v;
+  asm volatile("ld.global.L2::cache_hint.u8 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol));
+  return v;
+}
+template <bool KEEP, bool from_evidence, bool kMask>
 __device__ __forceinline__ RawNig fetch_nig(const float* __restrict__ evidence, const float* __restrict__ gamma,
                                             const float* __restrict__ nu, const float* __restrict__ alpha,
                                             const float* __restrict__ beta, const float* __restrict__ targets,
-                                            int e, unsigned long long pol) {
+                                            const unsigned char* __restrict__ mask, int e, unsigned long long pol) {
   RawNig r;
+  r.lab = true;
   if (KEEP) {
     if (from_evidence) r.v = ld_keep_f4(reinterpret_cast<const float4*>(evidence) + e, pol);
     else r.v = make_float4(ld_keep_f(gamma + e, pol), ld_keep_f(nu + e, pol), ld_keep_f(alpha + e, pol),
@@ -205,6 +220,10 @@ __device__ __forceinline__ RawNig fetch_nig(const float* __restrict__ evidence, 
     if (from_evidence) r.v = __ldcs(reinterpret_cast<const float4*>(evidence) + e);
     else r.v = make_float4(__ldcs(gamma + e), __ldcs(nu + e), __ldcs(alpha + e), __ldcs(beta + e));
     r.y = __ldcs(targets + e);
+  }
+  if (kMask) {
+    r.lab = (KEEP ? ld_keep_u8(mask + e, pol) : (unsigned)__ldcs(mask + e)) != 0u;
+    r.y = r.lab ? r.y : r.v.x;   // a select: the unlabelled target value never enters the math
   }
   return r;
 }
@@ -283,16 +302,19 @@ __device__ __forceinline__ StatsOut<V> stats_math(const NigT<V>& p, V y, float e
 // element indices are 32-bit inside the kernels (the entry points reject B*D >= 2^31 - grid slack)
 // from_evidence is a template parameter: as a runtime flag both load variants were emitted predicated, and the
 // predicated-off half still took ~10 issue slots per element
-template <bool KEEP, bool from_evidence, bool PIPE>
+// kMask: partially labelled batch (mask appended to the parameter list, so the plain instantiations keep their layout)
+template <bool KEEP, bool from_evidence, bool PIPE, bool kMask>
 __global__ void __launch_bounds__(LOSS_THREADS, PIPE ? LOSS_MIN_BLOCKS_PIPE : LOSS_MIN_BLOCKS) nig_loss_stats_kernel(
     const float* __restrict__ evidence, const float* __restrict__ gamma, const float* __restrict__ nu,
     const float* __restrict__ alpha, const float* __restrict__ beta, const float* __restrict__ targets,
     const float* __restrict__ bin_edges, float* __restrict__ stats, const NigPlanes planes, int nig_out, int total, int D,
-    float eps) {
+    float eps, const unsigned char* __restrict__ mask) {
   DEER_PDL_ENTRY();
+  constexpr int NRED = kMask ? 6 : 5;     // register sums reduced through shared memory (+ the labelled count)
+  constexpr int NRS = 30 + NRED;          // statistics written per dimension
   __shared__ float bins[3 * NBINS][LOSS_THREADS];  // private column per thread: conflict-free, no atomics
   __shared__ float sedges[NBINS + 1];
-  __shared__ float red[5][LOSS_THREADS];
+  __shared__ float red[NRED][LOSS_THREADS];
   const int tid = threadIdx.x;
   if (tid <= NBINS) sedges[tid] = bin_edges[tid];
 #pragma unroll
@@ -302,11 +324,17 @@ __global__ void __launch_bounds__(LOSS_THREADS, PIPE ? LOSS_MIN_BLOCKS_PIPE : LO
   const float log1eps = logf(1.f + eps);
   const bool eps_is_1e8 = eps == 1e-8f;
   P2 a_nll(0.f), a_reg(0.f), a_kla(0.f), a_klb(0.f), a_u(0.f);   // per-component partial sums, folded at the end
+  float a_n = 0.f;                                                 // kMask: labelled elements seen by this thread
   const unsigned long long pol = KEEP ? l2_evict_last_policy() : 0ull;
   const int stride = (int)gridDim.x * LOSS_THREADS;  // multiple of D -> dimension fixed per thread
-  auto tail = [&](float conf, float aerr, const NigT<float>& p, float alea, float epis, int e) {
+  // a statistic contribution, selected to 0 at an unlabelled element
+  auto keep = [&](auto v, auto m) {
+    if constexpr (kMask) return vsel(m, v, decltype(v)(0.f));
+    else return v;
+  };
+  auto tail = [&](float conf, float aerr, const NigT<float>& p, float alea, float epis, int e, bool lab) {
     const int k = ece_bin(conf, sedges);
-    if (k >= 0) {
+    if (k >= 0 && lab) {
       bins[k][tid] += 1.f;
       bins[NBINS + k][tid] += conf;
       bins[2 * NBINS + k][tid] += aerr;
@@ -326,26 +354,29 @@ __global__ void __launch_bounds__(LOSS_THREADS, PIPE ? LOSS_MIN_BLOCKS_PIPE : LO
     const NigT<P2> p = derive_nig<from_evidence>(P2(r0.v.x, r1.v.x), P2(r0.v.y, r1.v.y), P2(r0.v.z, r1.v.z),
                                                  P2(r0.v.w, r1.v.w));
     const StatsOut<P2> o = stats_math(p, P2(r0.y, r1.y), eps, inv_two_pi_eps, log1eps, eps_is_1e8, nig_out);
-    a_nll = a_nll + o.nll;
-    a_reg = a_reg + o.reg;
-    a_kla = a_kla + o.kla;
-    a_klb = a_klb + o.klb;
-    a_u = a_u + o.u;
+    const M2 m{r0.lab, r1.lab};
+    a_nll = a_nll + keep(o.nll, m);
+    a_reg = a_reg + keep(o.reg, m);
+    a_kla = a_kla + keep(o.kla, m);
+    a_klb = a_klb + keep(o.klb, m);
+    a_u = a_u + keep(o.u, m);
+    if constexpr (kMask) a_n += (r0.lab ? 1.f : 0.f) + (r1.lab ? 1.f : 0.f);
     NigT<float> q0, q1;
     q0.gamma = p.gamma.x; q0.nu = p.nu.x; q0.alpha = p.alpha.x; q0.beta = p.beta.x;
     q1.gamma = p.gamma.y; q1.nu = p.nu.y; q1.alpha = p.alpha.y; q1.beta = p.beta.y;
-    tail(o.conf.x, o.aerr.x, q0, o.alea.x, o.epis.x, e0);
-    tail(o.conf.y, o.aerr.y, q1, o.alea.y, o.epis.y, e1);
+    tail(o.conf.x, o.aerr.x, q0, o.alea.x, o.epis.x, e0, r0.lab);
+    tail(o.conf.y, o.aerr.y, q1, o.alea.y, o.epis.y, e1, r1.lab);
   };
   auto single = [&](const RawNig& r, int e) {
     const NigT<float> p = derive_nig<from_evidence>(r.v.x, r.v.y, r.v.z, r.v.w);
     const StatsOut<float> o = stats_math(p, r.y, eps, inv_two_pi_eps, log1eps, eps_is_1e8, nig_out);
-    a_nll.x += o.nll;
-    a_reg.x += o.reg;
-    a_kla.x += o.kla;
-    a_klb.x += o.klb;
-    a_u.x += o.u;
-    tail(o.conf, o.aerr, p, o.alea, o.epis, e);
+    a_nll.x += keep(o.nll, r.lab);
+    a_reg.x += keep(o.reg, r.lab);
+    a_kla.x += keep(o.kla, r.lab);
+    a_klb.x += keep(o.klb, r.lab);
+    a_u.x += keep(o.u, r.lab);
+    if constexpr (kMask) a_n += r.lab ? 1.f : 0.f;
+    tail(o.conf, o.aerr, p, o.alea, o.epis, e, r.lab);
   };
   int eb = (int)blockIdx.x * LOSS_THREADS + tid;
   if constexpr (PIPE) {
@@ -356,7 +387,8 @@ __global__ void __launch_bounds__(LOSS_THREADS, PIPE ? LOSS_MIN_BLOCKS_PIPE : LO
     if (have) {
 #pragma unroll
       for (int q = 0; q < LOSS_UNROLL; q++)
-        rr[q] = fetch_nig<KEEP, from_evidence>(evidence, gamma, nu, alpha, beta, targets, eb + q * stride, pol);
+        rr[q] = fetch_nig<KEEP, from_evidence, kMask>(evidence, gamma, nu, alpha, beta, targets, mask,
+                                                      eb + q * stride, pol);
     }
     while (have) {
       const int en = eb + LOSS_UNROLL * stride;
@@ -365,7 +397,8 @@ __global__ void __launch_bounds__(LOSS_THREADS, PIPE ? LOSS_MIN_BLOCKS_PIPE : LO
       if (more) {
 #pragma unroll
         for (int q = 0; q < LOSS_UNROLL; q++)
-          nx[q] = fetch_nig<KEEP, from_evidence>(evidence, gamma, nu, alpha, beta, targets, en + q * stride, pol);
+          nx[q] = fetch_nig<KEEP, from_evidence, kMask>(evidence, gamma, nu, alpha, beta, targets, mask,
+                                                        en + q * stride, pol);
       }
 #pragma unroll
       for (int q = 0; q < LOSS_UNROLL; q += 2) pair(rr[q], rr[q + 1], eb + q * stride, eb + (q + 1) * stride);
@@ -381,28 +414,30 @@ __global__ void __launch_bounds__(LOSS_THREADS, PIPE ? LOSS_MIN_BLOCKS_PIPE : LO
       RawNig rr[LOSS_UNROLL];
 #pragma unroll
       for (int q = 0; q < LOSS_UNROLL; q++)
-        rr[q] = fetch_nig<KEEP, from_evidence>(evidence, gamma, nu, alpha, beta, targets, eb + q * stride, pol);
+        rr[q] = fetch_nig<KEEP, from_evidence, kMask>(evidence, gamma, nu, alpha, beta, targets, mask,
+                                                      eb + q * stride, pol);
 #pragma unroll
       for (int q = 0; q < LOSS_UNROLL; q += 2) pair(rr[q], rr[q + 1], eb + q * stride, eb + (q + 1) * stride);
     }
   }
   for (; eb < total; eb += stride)
-    single(fetch_nig<KEEP, from_evidence>(evidence, gamma, nu, alpha, beta, targets, eb, pol), eb);
+    single(fetch_nig<KEEP, from_evidence, kMask>(evidence, gamma, nu, alpha, beta, targets, mask, eb, pol), eb);
   red[0][tid] = hsum(a_nll);
   red[1][tid] = hsum(a_reg);
   red[2][tid] = hsum(a_kla);
   red[3][tid] = hsum(a_klb);
   red[4][tid] = hsum(a_u);
+  if constexpr (kMask) red[NRED - 1][tid] = a_n;
   __syncthreads();
-  // thread (d, s) for s < 35 sums the columns of threads whose dimension is d (tid % D == d)
+  // thread (d, s) for s < NRS sums the columns of threads whose dimension is d (tid % D == d)
   const int first_e_dim = ((int)blockIdx.x * LOSS_THREADS) % D;
-  for (int w = tid; w < D * 35; w += LOSS_THREADS) {
-    const int d = w / 35, s = w % 35;
+  for (int w = tid; w < D * NRS; w += LOSS_THREADS) {
+    const int d = w / NRS, s = w % NRS;
     // threads t with (first_e_dim + t) % D == d
     int t0 = (d - first_e_dim) % D;
     if (t0 < 0) t0 += D;
     float acc = 0.f;
-    const float* src = s < 5 ? red[s] : bins[s - 5];
+    const float* src = s < 5 ? red[s] : (kMask && s == 35 ? red[NRED - 1] : bins[s - 5]);
     for (int t = t0; t < LOSS_THREADS; t += D) acc += src[t];
     if (acc != 0.f) atomicAdd(stats + d * NSTAT + s, acc);
   }
@@ -452,22 +487,50 @@ __device__ __forceinline__ GradOut<V> grad_math(const NigT<V>& p, V y, float eps
   return o;
 }
 
-template <bool from_evidence, bool PIPE>
+// kMask: the means of dimension d are over its N_d labelled elements (statistic 35; B_global is not used), the
+// cross-dimension term covers the dimensions with N_d > 0, and unlabelled elements get a zero gradient
+template <bool from_evidence, bool PIPE, bool kMask>
 __global__ void __launch_bounds__(LOSS_THREADS, PIPE ? LOSS_MIN_BLOCKS_PIPE : LOSS_MIN_BLOCKS) nig_loss_finish_kernel(
     const float* __restrict__ evidence, const float* __restrict__ gamma, const float* __restrict__ nu,
     const float* __restrict__ alpha, const float* __restrict__ beta, const float* __restrict__ targets,
     const float* __restrict__ bin_edges, const float* __restrict__ stats, const float* __restrict__ task_weights,
     float reg_w, float kl_w, float ece_w, float cross_w, float eps, int total_local, long long B_global, int D,
-    float grad_scale, float* __restrict__ losses, float* __restrict__ d_out) {
+    float grad_scale, float* __restrict__ losses, float* __restrict__ d_out, const unsigned char* __restrict__ mask,
+    float* __restrict__ counts) {
   DEER_PDL_ENTRY();
   __shared__ DimCoef coef[8];
   __shared__ float sedges[NBINS + 1];
   __shared__ float ubar[8];
+  __shared__ float sinvn[kMask ? 8 : 1];   // kMask: 1 / N_d, 0 for a dimension without labels
   const int tid = threadIdx.x;
   const float invN = 1.f / (float)B_global;
   if (tid <= NBINS) sedges[tid] = bin_edges[tid];
-  if (tid < D) ubar[tid] = stats[tid * NSTAT + 4] * invN;
+  if (tid < D) {
+    if constexpr (kMask) {
+      const float n = stats[tid * NSTAT + 35];
+      sinvn[tid] = n > 0.f ? 1.f / n : 0.f;
+      ubar[tid] = stats[tid * NSTAT + 4] * sinvn[tid];
+    } else {
+      ubar[tid] = stats[tid * NSTAT + 4] * invN;
+    }
+  }
   __syncthreads();
+  auto inv_n = [&](int d) -> float {
+    if constexpr (kMask) return sinvn[d];
+    else return invN;
+  };
+  auto present = [&](int d) -> bool {   // dimension d takes part in the cross-dimension term
+    if constexpr (kMask) return sinvn[d] > 0.f;
+    else return true;
+  };
+  auto num_pairs = [&]() -> int {   // pairs of dimensions in the cross-dimension term
+    int n = D;
+    if constexpr (kMask) {
+      n = 0;
+      for (int j = 0; j < D; j++) n += present(j) ? 1 : 0;
+    }
+    return n * (n - 1) / 2;
+  };
   __shared__ float ece_part[8][NBINS];
   if (tid < D * NBINS) {  // one thread per (dimension, bin): no serial chain of dependent global loads and divisions
     const int dd = tid / NBINS, k = tid % NBINS;
@@ -476,7 +539,7 @@ __global__ void __launch_bounds__(LOSS_THREADS, PIPE ? LOSS_MIN_BLOCKS_PIPE : LO
     float sg = 0.f, part = 0.f;
     if (cnt > 0.f) {
       const float diff = sc / cnt - (1.f - se / cnt);
-      part = (cnt * invN) * fabsf(diff);
+      part = (cnt * inv_n(dd)) * fabsf(diff);
       sg = diff > 0.f ? 1.f : (diff < 0.f ? -1.f : 0.f);
     }
     coef[dd].sign[k] = sg;
@@ -485,9 +548,9 @@ __global__ void __launch_bounds__(LOSS_THREADS, PIPE ? LOSS_MIN_BLOCKS_PIPE : LO
   if (tid < D) {
     float cs = 0.f;
     for (int j = 0; j < D; j++)
-      if (j != tid) cs += ubar[tid] - ubar[j];
-    const int npairs = D * (D - 1) / 2;
-    coef[tid].cross = npairs > 0 ? 2.f * cs / (float)npairs : 0.f;
+      if (j != tid && present(j)) cs += ubar[tid] - ubar[j];
+    const int npairs = num_pairs();
+    coef[tid].cross = (npairs > 0 && present(tid)) ? 2.f * cs / (float)npairs : 0.f;
     coef[tid].w = task_weights ? task_weights[tid] : 1.f;
   }
   __syncthreads();
@@ -496,21 +559,24 @@ __global__ void __launch_bounds__(LOSS_THREADS, PIPE ? LOSS_MIN_BLOCKS_PIPE : LO
       const float* st = stats + tid * NSTAT;
       float ece = 0.f;
       for (int k = 0; k < NBINS; k++) ece += ece_part[tid][k];
-      const float nll = st[0] * invN, reg = st[1] * invN;
-      const float kl = st[2] * invN + 0.1f * st[3] * invN;
+      const float in = inv_n(tid);   // a dimension without labels: every sum is 0, and so is every entry
+      const float nll = st[0] * in, reg = st[1] * in;
+      const float kl = st[2] * in + 0.1f * st[3] * in;
       float* L = losses + tid * 5;
       L[0] = nll + reg_w * reg + kl_w * kl + ece_w * ece;
       L[1] = nll;
       L[2] = reg;
       L[3] = kl;
       L[4] = ece;
+      if (kMask && counts) counts[tid] = st[35];
     }
     __syncthreads();
     if (tid == 0) {
       float cd = 0.f;
       for (int i = 0; i < D; i++)
-        for (int j = i + 1; j < D; j++) cd += (ubar[i] - ubar[j]) * (ubar[i] - ubar[j]);
-      const int npairs = D * (D - 1) / 2;
+        for (int j = i + 1; j < D; j++)
+          if (present(i) && present(j)) cd += (ubar[i] - ubar[j]) * (ubar[i] - ubar[j]);
+      const int npairs = num_pairs();
       if (npairs > 0) cd /= (float)npairs;
       float tot = 0.f;
       for (int i = 0; i < D; i++) tot += coef[i].w * losses[i * 5];
@@ -525,12 +591,12 @@ __global__ void __launch_bounds__(LOSS_THREADS, PIPE ? LOSS_MIN_BLOCKS_PIPE : LO
   const int stride = (int)gridDim.x * LOSS_THREADS;  // multiple of D: the dimension is fixed per thread
   const int d = ((int)blockIdx.x * LOSS_THREADS + tid) % D;
   const float w = coef[d].w;
-  const float base_w = grad_scale * invD * invN * w;   // task weight folded into the output scale
+  const float base_w = grad_scale * invD * inv_n(d) * w;   // task weight folded into the output scale
   const bool eps_is_1e8 = eps == 1e-8f;
   // cross-dimension term enters UNWEIGHTED by the task weight: pre-divide by w where w != 0 (w == 0: term dropped,
   // handled by the separate scale below)
   const float cross_c = (cross_w > 0.f && D > 1) ? cross_w * coef[d].cross : 0.f;
-  const float base = grad_scale * invD * invN;
+  const float base = grad_scale * invD * inv_n(d);
   const float ece_on = ece_w > 0.f ? ece_w : 0.f;
   const float* __restrict__ sgn = coef[d].sign;
   // ECE bin sign of one element (scalar: a bin search and a shared-memory lookup), pre-multiplied by the ECE weight
@@ -539,7 +605,7 @@ __global__ void __launch_bounds__(LOSS_THREADS, PIPE ? LOSS_MIN_BLOCKS_PIPE : LO
     return k >= 0 ? sgn[max(k, 0)] * ece_on : 0.f;
   };
   // ECE and cross-dimension corrections, task weight, chain rule back to the evidence: value-typed like the rest
-  auto finish = [&](auto g, const auto& p, auto sg) {
+  auto finish = [&](auto g, const auto& p, auto sg, auto m) {
     using V = decltype(g.dg);
     if (ece_on > 0.f) {  // uniform
       const V t = V(0.f) - sg * (g.conf * g.conf) * g.rden;  // sg * dconf/du * 1/den
@@ -560,6 +626,12 @@ __global__ void __launch_bounds__(LOSS_THREADS, PIPE ? LOSS_MIN_BLOCKS_PIPE : LO
       oz = oz * p.sa;
       ow = ow * p.sb;
     }
+    if constexpr (kMask) {   // exactly 0 at an unlabelled element
+      ox = vsel(m, ox, V(0.f));
+      oy = vsel(m, oy, V(0.f));
+      oz = vsel(m, oz, V(0.f));
+      ow = vsel(m, ow, V(0.f));
+    }
     g.dg = ox; g.dn = oy; g.da = oz; g.db = ow;
     return g;
   };
@@ -568,7 +640,7 @@ __global__ void __launch_bounds__(LOSS_THREADS, PIPE ? LOSS_MIN_BLOCKS_PIPE : LO
                                                  P2(r0.v.w, r1.v.w));
     GradOut<P2> g = grad_math(p, P2(r0.y, r1.y), eps, log1eps, reg_w, kl_w);
     const P2 sg = ece_on > 0.f ? P2(bin_sign(g.conf.x), bin_sign(g.conf.y)) : P2(0.f);
-    g = finish(g, p, sg);
+    g = finish(g, p, sg, M2{r0.lab, r1.lab});
     __stcs(reinterpret_cast<float4*>(d_out) + e0, make_float4(g.dg.x, g.dn.x, g.da.x, g.db.x));
     __stcs(reinterpret_cast<float4*>(d_out) + e1, make_float4(g.dg.y, g.dn.y, g.da.y, g.db.y));
   };
@@ -576,7 +648,7 @@ __global__ void __launch_bounds__(LOSS_THREADS, PIPE ? LOSS_MIN_BLOCKS_PIPE : LO
     const NigT<float> p = derive_nig<from_evidence>(r.v.x, r.v.y, r.v.z, r.v.w);
     GradOut<float> g = grad_math(p, r.y, eps, log1eps, reg_w, kl_w);
     const float sg = ece_on > 0.f ? bin_sign(g.conf) : 0.f;
-    g = finish(g, p, sg);
+    g = finish(g, p, sg, r.lab);
     __stcs(reinterpret_cast<float4*>(d_out) + e, make_float4(g.dg, g.dn, g.da, g.db));
   };
   int eb = (int)blockIdx.x * LOSS_THREADS + tid;
@@ -586,7 +658,8 @@ __global__ void __launch_bounds__(LOSS_THREADS, PIPE ? LOSS_MIN_BLOCKS_PIPE : LO
     if (have) {
 #pragma unroll
       for (int q = 0; q < LOSS_UNROLL; q++)
-        rr[q] = fetch_nig<false, from_evidence>(evidence, gamma, nu, alpha, beta, targets, eb + q * stride, 0ull);
+        rr[q] = fetch_nig<false, from_evidence, kMask>(evidence, gamma, nu, alpha, beta, targets, mask,
+                                                       eb + q * stride, 0ull);
     }
     while (have) {
       const int en = eb + LOSS_UNROLL * stride;
@@ -595,7 +668,8 @@ __global__ void __launch_bounds__(LOSS_THREADS, PIPE ? LOSS_MIN_BLOCKS_PIPE : LO
       if (more) {
 #pragma unroll
         for (int q = 0; q < LOSS_UNROLL; q++)
-          nx[q] = fetch_nig<false, from_evidence>(evidence, gamma, nu, alpha, beta, targets, en + q * stride, 0ull);
+          nx[q] = fetch_nig<false, from_evidence, kMask>(evidence, gamma, nu, alpha, beta, targets, mask,
+                                                         en + q * stride, 0ull);
       }
 #pragma unroll
       for (int q = 0; q < LOSS_UNROLL; q += 2) pair(rr[q], rr[q + 1], eb + q * stride, eb + (q + 1) * stride);
@@ -611,13 +685,14 @@ __global__ void __launch_bounds__(LOSS_THREADS, PIPE ? LOSS_MIN_BLOCKS_PIPE : LO
       RawNig rr[LOSS_UNROLL];
 #pragma unroll
       for (int q = 0; q < LOSS_UNROLL; q++)
-        rr[q] = fetch_nig<false, from_evidence>(evidence, gamma, nu, alpha, beta, targets, eb + q * stride, 0ull);
+        rr[q] = fetch_nig<false, from_evidence, kMask>(evidence, gamma, nu, alpha, beta, targets, mask,
+                                                       eb + q * stride, 0ull);
 #pragma unroll
       for (int q = 0; q < LOSS_UNROLL; q += 2) pair(rr[q], rr[q + 1], eb + q * stride, eb + (q + 1) * stride);
     }
   }
   for (; eb < total_local; eb += stride)
-    single(fetch_nig<false, from_evidence>(evidence, gamma, nu, alpha, beta, targets, eb, 0ull), eb);
+    single(fetch_nig<false, from_evidence, kMask>(evidence, gamma, nu, alpha, beta, targets, mask, eb, 0ull), eb);
 }
 
 // ------------------------------------------------------------------ stand-alone head
@@ -759,6 +834,85 @@ static int stream_grid(long long n, int threads) {
 
 int g_nig_pipe = 1;   // DEER_OPT_NIG_PIPELINE
 
+// launchers shared by the plain and the mask entries (kMask: target_mask [B,D] bytes, nonzero = labelled)
+template <bool kMask>
+static int nig_loss_stats_launch(const float* evidence, const float* gamma, const float* nu, const float* alpha,
+                                 const float* beta, const float* targets, const unsigned char* mask,
+                                 const float* bin_edges, float* stats, float* nig_out, long long B, int D,
+                                 int from_evidence, float eps, void* stream) {
+  DEER_CHECK_ARG(targets && bin_edges && stats && B > 0, "nig_loss_stats: bad args");
+  DEER_CHECK_ARG(from_evidence ? evidence != nullptr : (gamma && nu && alpha && beta), "nig_loss_stats: inputs");
+  if (D < 1 || D > 8 || LOSS_THREADS % D != 0) {
+    set_error("nig_loss_stats: D=%d unsupported (need a divisor of %d, <=8)", D, LOSS_THREADS);
+    return DEER_ERR_UNSUPPORTED;
+  }
+  const long long total = B * D;
+  if (total > DEER_NIG_MAX_ELEMENTS) {
+    set_error("nig_loss_stats: B*D=%lld exceeds %lld", total, (long long)DEER_NIG_MAX_ELEMENTS);
+    return DEER_ERR_UNSUPPORTED;
+  }
+  NigPlanes planes;
+  for (int i = 0; i < 7; i++) planes.p[i] = nig_out ? nig_out + (long long)i * total : nullptr;
+  const int has_out = nig_out != nullptr;
+  // operands (20 B per element) small enough to stay in the 126 MB L2 between the two passes?
+  const bool keep = total * 20 <= (long long)DEER_NIG_L2_KEEP_BYTES;
+#define DEER_NIG_STATS_GO(K, FE, PP)                                                                                  \
+  DEER_LAUNCH((nig_loss_stats_kernel<K, FE, PP, kMask>),                                                               \
+              resident_grid(nig_loss_stats_kernel<K, FE, PP, kMask>, total, LOSS_THREADS), LOSS_THREADS, 0, stream,   \
+              evidence, gamma, nu, alpha, beta, targets, bin_edges, stats, planes, has_out, (int)total, D, eps, mask)
+#define DEER_NIG_STATS_GO2(K, FE)            \
+  do {                                       \
+    if (g_nig_pipe) DEER_NIG_STATS_GO(K, FE, true); \
+    else DEER_NIG_STATS_GO(K, FE, false);    \
+  } while (0)
+  if (keep) {
+    if (from_evidence) DEER_NIG_STATS_GO2(true, true);
+    else DEER_NIG_STATS_GO2(true, false);
+  } else {
+    if (from_evidence) DEER_NIG_STATS_GO2(false, true);
+    else DEER_NIG_STATS_GO2(false, false);
+  }
+#undef DEER_NIG_STATS_GO2
+#undef DEER_NIG_STATS_GO
+  return DEER_OK;
+}
+
+template <bool kMask>
+static int nig_loss_finish_launch(const float* evidence, const float* gamma, const float* nu, const float* alpha,
+                                  const float* beta, const float* targets, const unsigned char* mask,
+                                  const float* bin_edges, const float* stats, const float* task_weights, float reg_w,
+                                  float kl_w, float ece_w, float cross_w, float eps, long long B_local,
+                                  long long B_global, int D, int from_evidence, float grad_scale, float* losses,
+                                  float* d_out, float* counts, void* stream) {
+  DEER_CHECK_ARG(targets && bin_edges && stats && B_local > 0, "nig_loss_finish: bad args");
+  DEER_CHECK_ARG(from_evidence ? evidence != nullptr : (gamma && nu && alpha && beta), "nig_loss_finish: inputs");
+  DEER_CHECK_ARG(losses || d_out, "nig_loss_finish: nothing to do");
+  if (D < 1 || D > 8) {
+    set_error("nig_loss_finish: D=%d unsupported", D);
+    return DEER_ERR_UNSUPPORTED;
+  }
+  const long long total = B_local * D;
+  if (total > DEER_NIG_MAX_ELEMENTS) {
+    set_error("nig_loss_finish: B*D=%lld exceeds %lld", total, (long long)DEER_NIG_MAX_ELEMENTS);
+    return DEER_ERR_UNSUPPORTED;
+  }
+#define DEER_NIG_FINISH_GO(FE, PP)                                                                                    \
+  DEER_LAUNCH((nig_loss_finish_kernel<FE, PP, kMask>),                                                                 \
+              resident_grid(nig_loss_finish_kernel<FE, PP, kMask>, total, LOSS_THREADS), LOSS_THREADS, 0, stream,     \
+              evidence, gamma, nu, alpha, beta, targets, bin_edges, stats, task_weights, reg_w, kl_w, ece_w, cross_w, \
+              eps, (int)total, B_global, D, grad_scale, losses, d_out, mask, counts)
+  if (from_evidence) {
+    if (g_nig_pipe) DEER_NIG_FINISH_GO(true, true);
+    else DEER_NIG_FINISH_GO(true, false);
+  } else {
+    if (g_nig_pipe) DEER_NIG_FINISH_GO(false, true);
+    else DEER_NIG_FINISH_GO(false, false);
+  }
+#undef DEER_NIG_FINISH_GO
+  return DEER_OK;
+}
+
+
 }  // namespace deer
 
 using namespace deer;
@@ -786,41 +940,18 @@ int deer_nig_head_bwd(const float* evidence, const float* dmu, const float* dnu,
 int deer_nig_loss_stats(const float* evidence, const float* gamma, const float* nu, const float* alpha,
                         const float* beta, const float* targets, const float* bin_edges, float* stats, float* nig_out,
                         long long B, int D, int from_evidence, float eps, void* stream) {
-  DEER_CHECK_ARG(targets && bin_edges && stats && B > 0, "nig_loss_stats: bad args");
-  DEER_CHECK_ARG(from_evidence ? evidence != nullptr : (gamma && nu && alpha && beta), "nig_loss_stats: inputs");
-  if (D < 1 || D > 8 || LOSS_THREADS % D != 0) {
-    set_error("nig_loss_stats: D=%d unsupported (need a divisor of %d, <=8)", D, LOSS_THREADS);
-    return DEER_ERR_UNSUPPORTED;
-  }
-  const long long total = B * D;
-  if (total > DEER_NIG_MAX_ELEMENTS) {
-    set_error("nig_loss_stats: B*D=%lld exceeds %lld", total, (long long)DEER_NIG_MAX_ELEMENTS);
-    return DEER_ERR_UNSUPPORTED;
-  }
-  NigPlanes planes;
-  for (int i = 0; i < 7; i++) planes.p[i] = nig_out ? nig_out + (long long)i * total : nullptr;
-  const int has_out = nig_out != nullptr;
-  // operands (20 B per element) small enough to stay in the 126 MB L2 between the two passes?
-  const bool keep = total * 20 <= (long long)DEER_NIG_L2_KEEP_BYTES;
-#define DEER_NIG_STATS_GO(K, FE, PP)                                                                                  \
-  DEER_LAUNCH((nig_loss_stats_kernel<K, FE, PP>), resident_grid(nig_loss_stats_kernel<K, FE, PP>, total, LOSS_THREADS), \
-              LOSS_THREADS, 0, stream, evidence, gamma, nu, alpha, beta, targets, bin_edges, stats, planes, has_out,  \
-              (int)total, D, eps)
-#define DEER_NIG_STATS_GO2(K, FE)            \
-  do {                                       \
-    if (g_nig_pipe) DEER_NIG_STATS_GO(K, FE, true); \
-    else DEER_NIG_STATS_GO(K, FE, false);    \
-  } while (0)
-  if (keep) {
-    if (from_evidence) DEER_NIG_STATS_GO2(true, true);
-    else DEER_NIG_STATS_GO2(true, false);
-  } else {
-    if (from_evidence) DEER_NIG_STATS_GO2(false, true);
-    else DEER_NIG_STATS_GO2(false, false);
-  }
-#undef DEER_NIG_STATS_GO2
-#undef DEER_NIG_STATS_GO
-  return DEER_OK;
+  return nig_loss_stats_launch<false>(evidence, gamma, nu, alpha, beta, targets, nullptr, bin_edges, stats, nig_out, B,
+                                      D, from_evidence, eps, stream);
+}
+
+int deer_nig_loss_stats_mask(const float* evidence, const float* gamma, const float* nu, const float* alpha,
+                             const float* beta, const float* targets, const void* target_mask, const float* bin_edges,
+                             float* stats, float* nig_out, long long B, int D, int from_evidence, float eps,
+                             void* stream) {
+  DEER_CHECK_ARG(target_mask, "nig_loss_stats_mask: target_mask");
+  return nig_loss_stats_launch<true>(evidence, gamma, nu, alpha, beta, targets,
+                                     static_cast<const unsigned char*>(target_mask), bin_edges, stats, nig_out, B, D,
+                                     from_evidence, eps, stream);
 }
 
 int deer_nig_loss_finish(const float* evidence, const float* gamma, const float* nu, const float* alpha,
@@ -828,31 +959,24 @@ int deer_nig_loss_finish(const float* evidence, const float* gamma, const float*
                          const float* task_weights, float reg_w, float kl_w, float ece_w, float cross_w, float eps,
                          long long B_local, long long B_global, int D, int from_evidence, float grad_scale,
                          float* losses, float* d_out, void* stream) {
-  DEER_CHECK_ARG(targets && bin_edges && stats && B_local > 0 && B_global >= B_local, "nig_loss_finish: bad args");
-  DEER_CHECK_ARG(from_evidence ? evidence != nullptr : (gamma && nu && alpha && beta), "nig_loss_finish: inputs");
-  DEER_CHECK_ARG(losses || d_out, "nig_loss_finish: nothing to do");
-  if (D < 1 || D > 8) {
-    set_error("nig_loss_finish: D=%d unsupported", D);
-    return DEER_ERR_UNSUPPORTED;
-  }
-  const long long total = B_local * D;
-  if (total > DEER_NIG_MAX_ELEMENTS) {
-    set_error("nig_loss_finish: B*D=%lld exceeds %lld", total, (long long)DEER_NIG_MAX_ELEMENTS);
-    return DEER_ERR_UNSUPPORTED;
-  }
-#define DEER_NIG_FINISH_GO(FE, PP)                                                                                    \
-  DEER_LAUNCH((nig_loss_finish_kernel<FE, PP>), resident_grid(nig_loss_finish_kernel<FE, PP>, total, LOSS_THREADS),   \
-              LOSS_THREADS, 0, stream, evidence, gamma, nu, alpha, beta, targets, bin_edges, stats, task_weights,     \
-              reg_w, kl_w, ece_w, cross_w, eps, (int)total, B_global, D, grad_scale, losses, d_out)
-  if (from_evidence) {
-    if (g_nig_pipe) DEER_NIG_FINISH_GO(true, true);
-    else DEER_NIG_FINISH_GO(true, false);
-  } else {
-    if (g_nig_pipe) DEER_NIG_FINISH_GO(false, true);
-    else DEER_NIG_FINISH_GO(false, false);
-  }
-#undef DEER_NIG_FINISH_GO
-  return DEER_OK;
+  DEER_CHECK_ARG(B_global >= B_local, "nig_loss_finish: bad args");
+  return nig_loss_finish_launch<false>(evidence, gamma, nu, alpha, beta, targets, nullptr, bin_edges, stats,
+                                       task_weights, reg_w, kl_w, ece_w, cross_w, eps, B_local, B_global, D,
+                                       from_evidence, grad_scale, losses, d_out, nullptr, stream);
+}
+
+int deer_nig_loss_finish_mask(const float* evidence, const float* gamma, const float* nu, const float* alpha,
+                              const float* beta, const float* targets, const void* target_mask,
+                              const float* bin_edges, const float* stats, const float* task_weights, float reg_w,
+                              float kl_w, float ece_w, float cross_w, float eps, long long B_local, int D,
+                              int from_evidence, float grad_scale, float* losses, float* d_out, float* counts,
+                              void* stream) {
+  DEER_CHECK_ARG(target_mask, "nig_loss_finish_mask: target_mask");
+  DEER_CHECK_ARG(losses || !counts, "nig_loss_finish_mask: counts are written with the losses");
+  return nig_loss_finish_launch<true>(evidence, gamma, nu, alpha, beta, targets,
+                                      static_cast<const unsigned char*>(target_mask), bin_edges, stats, task_weights,
+                                      reg_w, kl_w, ece_w, cross_w, eps, B_local, B_local, D, from_evidence, grad_scale,
+                                      losses, d_out, counts, stream);
 }
 
 int deer_amini_loss(const float* mu, const float* nu, const float* alpha, const float* beta, const float* targets,

@@ -4,7 +4,10 @@ Wire format (reference: src/data/preprocessing.py:461-491 collate dict, src/mode
 the driver's synthetic loader yields 4-tuples, experiments/run_multimodal_deer.py:329-349):
 
     {"audio_features", "video_features", "text_features", "targets"[, "attention_mask", "linguistic_features",
-     "dataset_id"]}           or           (audio, video, text, targets)
+     "target_mask", "dataset_id"]}           or           (audio, video, text, targets)
+
+"target_mask" (the targets' shape, bool / uint8, nonzero = labelled) marks the targets a partially labelled batch
+has; it keeps its dtype on the device.
 
 `DevicePrefetcher` turns any iterable of such HOST batches into device batches whose H2D copies overlap the compute of
 the previous step: `depth` rotating sets of STATIC device buffers per batch signature (static addresses, so the
@@ -19,7 +22,7 @@ from typing import Dict, Iterable, Iterator, Optional
 import torch
 
 BATCH_KEYS = ("audio_features", "video_features", "text_features", "targets")
-OPTIONAL_KEYS = ("attention_mask", "linguistic_features", "dataset_id")
+OPTIONAL_KEYS = ("attention_mask", "linguistic_features", "target_mask", "dataset_id")
 
 
 def as_batch_dict(batch) -> Dict[str, torch.Tensor]:

@@ -5,6 +5,12 @@ synchronises with the host (the reference does 10 host syncs per dimension in th
 
 Differentiability: `total_loss` carries the gradient; the per-term entries are detached views of the same device
 vector (the reference trainer only ever back-propagates total_loss, training.py:216).
+
+Partially labelled batches: every `forward` takes `target_mask` (bool / uint8 CUDA tensor of the targets' shape,
+nonzero = labelled).  Each dimension's terms are then the reference's on that dimension's labelled entries alone, the
+cross-dimension term averages over the dimensions that have labels, unlabelled target values (NaN, Inf, anything) are
+never used and get an exactly-zero gradient, and the output gains `{dim}_num_labeled` (detached 0-d tensors).  Without
+a mask nothing changes; in particular a NaN target still makes the loss NaN.
 """
 from __future__ import annotations
 
@@ -14,6 +20,7 @@ import torch
 import torch.nn as nn
 
 from . import ops
+from ._lib import DeerError
 from .deer import EVIDENCE_KEY
 
 _TERMS = ("total_loss", "nll_loss", "reg_loss", "kl_loss", "ece_loss")
@@ -53,7 +60,11 @@ class DEERLoss(nn.Module):
         super().__init__()
         self.reg_weight, self.kl_weight, self.ece_weight, self.epsilon = reg_weight, kl_weight, ece_weight, epsilon
 
-    def forward(self, predictions: Dict[str, torch.Tensor], targets: torch.Tensor) -> Dict[str, torch.Tensor]:
+    def forward(self, predictions: Dict[str, torch.Tensor], targets: torch.Tensor,
+                target_mask: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
+        if target_mask is not None and tuple(target_mask.shape) != tuple(targets.shape):
+            raise DeerError(f"deer_b200: `target_mask` must have the targets' shape {tuple(targets.shape)}, got "
+                            f"{tuple(target_mask.shape)}")
         gamma = _pick(predictions, "gamma", "mu")
         nu = _pick(predictions, "nu", "lambda")
         alpha, beta = predictions.get("alpha"), predictions.get("beta")
@@ -67,12 +78,19 @@ class DEERLoss(nn.Module):
             gamma, nu, alpha, beta, targets = (t.unsqueeze(-1) for t in (gamma, nu, alpha, beta, targets))
         B = gamma.shape[0]
         # the reference flattens [B,num_dims] into ONE population for the means and the ECE bins (losses.py:150,201)
+        # (the mask is flattened the same way)
         flat = [t.reshape(-1, 1) for t in (gamma, nu, alpha, beta)]
         l = ops.multitask_loss(*flat, targets.reshape(-1, 1),
-                               weights=(self.reg_weight, self.kl_weight, self.ece_weight, 0.0), eps=self.epsilon)
+                               weights=(self.reg_weight, self.kl_weight, self.ece_weight, 0.0), eps=self.epsilon,
+                               target_mask=None if target_mask is None else target_mask.reshape(-1, 1))
+        counts = None
+        if target_mask is not None:
+            l, counts = l
         out = {"total_loss": l[6]}                      # D=1: [tot,nll,reg,kl,ece, cross, total/1]
         d = l.detach()
         out.update({"nll_loss": d[1], "reg_loss": d[2], "kl_loss": d[3], "ece_loss": d[4], "batch_size": B})
+        if counts is not None:
+            out["num_labeled"] = counts[0]
         return out
 
 
@@ -94,12 +112,14 @@ class MultiTaskDEERLoss(nn.Module):
         tw = [float(self.task_weights[d]) for d in self.emotion_dims]
         return None if all(w == 1.0 for w in tw) else tw
 
-    def forward(self, predictions: Dict[str, torch.Tensor], targets: torch.Tensor) -> Dict[str, torch.Tensor]:
+    def forward(self, predictions: Dict[str, torch.Tensor], targets: torch.Tensor,
+                target_mask: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
         w, eps = self._weights()
         D = self.num_dims
         ev = predictions.get(EVIDENCE_KEY)
         if ev is not None and ev.shape[1] == D:
-            _, l = ops.fused_head_loss(ev, targets, w, eps, self._task_weight_list())
+            r = ops.fused_head_loss(ev, targets, w, eps, self._task_weight_list(), target_mask=target_mask)
+            l = r[1]
         else:
             cols = {k: [] for k in "gnab"}
             for d in self.emotion_dims:
@@ -108,14 +128,18 @@ class MultiTaskDEERLoss(nn.Module):
                 a, b = predictions[f"{d}_alpha"], predictions[f"{d}_beta"]
                 for key, t in zip("gnab", (g, n, a, b)):
                     cols[key].append(_as_col(t))
-            l = ops.multitask_loss(_gather(cols["g"]), _gather(cols["n"]), _gather(cols["a"]), _gather(cols["b"]),
-                                   targets, w, eps, self._task_weight_list())
+            r = ops.multitask_loss(_gather(cols["g"]), _gather(cols["n"]), _gather(cols["a"]), _gather(cols["b"]),
+                                   targets, w, eps, self._task_weight_list(), target_mask=target_mask)
+            l = r if target_mask is None else r[0]
+        counts = None if target_mask is None else r[-1]
         det = l.detach()
         out = {}
         for i, d in enumerate(self.emotion_dims):
             for j, term in enumerate(_TERMS):
                 out[f"{d}_{term}"] = det[5 * i + j]
             out[f"{d}_batch_size"] = targets.shape[0]
+            if counts is not None:
+                out[f"{d}_num_labeled"] = counts[i]
         if self.cross_dim_weight > 0 and D > 1:
             out["cross_dim_loss"] = det[5 * D]
         out["total_loss"] = l[5 * D + 1]
@@ -133,8 +157,8 @@ class CombinedDEERLoss(MultiTaskDEERLoss):
         self.deer_weight, self.uncertainty_weight, self.calibration_weight = (deer_weight, uncertainty_weight,
                                                                               calibration_weight)
 
-    def forward(self, predictions, targets):
-        out = super().forward(predictions, targets)
+    def forward(self, predictions, targets, target_mask=None):
+        out = super().forward(predictions, targets, target_mask)
         out["deer_loss"] = out["total_loss"]
         if self.deer_weight != 1.0:
             out["total_loss"] = out["total_loss"] * self.deer_weight

@@ -2172,16 +2172,39 @@ def ece_edges(device):
     return _edges_cache[key]
 
 
+def _target_mask(target_mask, t: torch.Tensor) -> torch.Tensor:
+    """Host-side checks of a target mask against targets `t` [B,D] (shape, dtype, device; the values are never read
+    here, so a step with a mask stays graph-capturable)."""
+    if not isinstance(target_mask, torch.Tensor) or not target_mask.is_cuda or target_mask.device != t.device:
+        raise _lib.DeerError(f"deer_b200: `target_mask` must be a CUDA tensor on {t.device}")
+    if target_mask.dtype not in (torch.bool, torch.uint8):
+        raise _lib.DeerError(f"deer_b200: `target_mask` must be bool or uint8, got {target_mask.dtype}")
+    if tuple(target_mask.shape) != tuple(t.shape):
+        raise _lib.DeerError(f"deer_b200: `target_mask` must have the targets' shape {tuple(t.shape)}, got "
+                             f"{tuple(target_mask.shape)}")
+    return target_mask.contiguous()
+
+
 def nig_loss_raw(evidence, params, targets, *, weights=(0.1, 0.01, 0.05, 0.05), eps=1e-8, task_weights=None,
-                 want_nig=False, want_grad=True, grad_scale=1.0, stats_hook=None, global_batch=None):
+                 want_nig=False, want_grad=True, grad_scale=1.0, stats_hook=None, global_batch=None, target_mask=None,
+                 counts=None):
     """Fused DEER multitask loss on either raw evidence [B,D,4] or params=(gamma,nu,alpha,beta) each [B,D].
 
     Returns (losses [5D+2], grad, nig_out [7,B,D] or None, stats [D,40]).  `stats_hook(stats)` runs between the two
-    phases (the data-parallel trainer all-reduces the statistics there)."""
+    phases (the data-parallel trainer all-reduces the statistics there).
+
+    `target_mask` [B,D] (bool / uint8, CUDA; nonzero = labelled): partially labelled batch.  Each dimension's terms
+    are means over its N_d labelled entries (N_d from the statistics, so after `stats_hook` it is the global count and
+    `global_batch` is not used), the cross-dimension term covers the dimensions with N_d > 0, a dimension without labels
+    has five 0 loss entries, and the gradient is exactly 0 at unlabelled entries, whatever their target values.
+    `counts` (float32 [D], mask only) receives N_d."""
     from_ev = evidence is not None
     t = _req(targets, "targets").contiguous()
     B, D = t.shape
     dev = t.device
+    m = None if target_mask is None else _target_mask(target_mask, t)
+    if counts is not None and (m is None or _req(counts, "counts").shape != (D,)):
+        raise _lib.DeerError(f"deer_b200: `counts` is a float32 [{D}] output of the target-mask path")
     if from_ev:
         e = _req(evidence, "evidence").contiguous()
         g = n = a = b = None
@@ -2191,63 +2214,93 @@ def nig_loss_raw(evidence, params, targets, *, weights=(0.1, 0.01, 0.05, 0.05), 
     stats = zeros_scratch((D, 40), dev)
     nig_out = torch.empty((7, B, D), device=dev, dtype=torch.float32) if want_nig else None
     edges = ece_edges(dev)
-    call("deer_nig_loss_stats", ptr(e), ptr(g), ptr(n), ptr(a), ptr(b), ptr(t), ptr(edges), ptr(stats), ptr(nig_out),
-         B, D, int(from_ev), float(eps))
+    if m is None:
+        call("deer_nig_loss_stats", ptr(e), ptr(g), ptr(n), ptr(a), ptr(b), ptr(t), ptr(edges), ptr(stats),
+             ptr(nig_out), B, D, int(from_ev), float(eps))
+    else:
+        call("deer_nig_loss_stats_mask", ptr(e), ptr(g), ptr(n), ptr(a), ptr(b), ptr(t), m.data_ptr(), ptr(edges),
+             ptr(stats), ptr(nig_out), B, D, int(from_ev), float(eps))
     if stats_hook is not None:
         stats_hook(stats)
     losses = torch.empty(5 * D + 2, device=dev, dtype=torch.float32)
     grad = torch.empty((B, D, 4), device=dev, dtype=torch.float32) if want_grad else None
     tw = None if task_weights is None else torch.as_tensor(task_weights, dtype=torch.float32, device=dev)
     rw, kw, ew, cw = weights
-    call("deer_nig_loss_finish", ptr(e), ptr(g), ptr(n), ptr(a), ptr(b), ptr(t), ptr(edges), ptr(stats), ptr(tw),
-         float(rw), float(kw), float(ew), float(cw), float(eps), B, int(global_batch or B), D, int(from_ev),
-         float(grad_scale), ptr(losses), ptr(grad))
+    if m is None:
+        call("deer_nig_loss_finish", ptr(e), ptr(g), ptr(n), ptr(a), ptr(b), ptr(t), ptr(edges), ptr(stats), ptr(tw),
+             float(rw), float(kw), float(ew), float(cw), float(eps), B, int(global_batch or B), D, int(from_ev),
+             float(grad_scale), ptr(losses), ptr(grad))
+    else:
+        call("deer_nig_loss_finish_mask", ptr(e), ptr(g), ptr(n), ptr(a), ptr(b), ptr(t), m.data_ptr(), ptr(edges),
+             ptr(stats), ptr(tw), float(rw), float(kw), float(ew), float(cw), float(eps), B, D, int(from_ev),
+             float(grad_scale), ptr(losses), ptr(grad), ptr(counts))
     return losses, grad, nig_out, stats
+
+
+def _mask_counts(target_mask, targets):
+    """The [D] output for N_d when a target mask is given (None otherwise)."""
+    if target_mask is None:
+        return None
+    return torch.empty(targets.shape[-1], device=targets.device, dtype=torch.float32)
 
 
 class _MultiTaskLoss(torch.autograd.Function):
     """losses.MultiTaskDEERLoss on contiguous [B,D] NIG parameter arrays.  Only `total` carries gradient."""
 
     @staticmethod
-    def forward(ctx, gamma, nu, alpha, beta, targets, weights, eps, task_weights):
+    def forward(ctx, gamma, nu, alpha, beta, targets, weights, eps, task_weights, target_mask=None):
+        counts = _mask_counts(target_mask, targets)
         losses, grad, _, _ = nig_loss_raw(None, (gamma, nu, alpha, beta), targets, weights=weights, eps=eps,
-                                          task_weights=task_weights)
+                                          task_weights=task_weights, target_mask=target_mask, counts=counts)
         ctx.save_for_backward(grad)
-        return losses
+        if counts is None:
+            return losses
+        ctx.mark_non_differentiable(counts)
+        return losses, counts
 
     @staticmethod
-    def backward(ctx, dlosses):
+    def backward(ctx, dlosses, *_dcounts):
         (grad,) = ctx.saved_tensors  # [B,D,4] = d total / d(gamma,nu,alpha,beta)
         D = grad.shape[1]
         s = dlosses[5 * D + 1]
         g = grad * s
-        return g[..., 0], g[..., 1], g[..., 2], g[..., 3], None, None, None, None
+        return g[..., 0], g[..., 1], g[..., 2], g[..., 3], None, None, None, None, None
 
 
-def multitask_loss(gamma, nu, alpha, beta, targets, weights=(0.1, 0.01, 0.05, 0.05), eps=1e-8, task_weights=None):
-    return _MultiTaskLoss.apply(gamma, nu, alpha, beta, targets, weights, eps, task_weights)
+def multitask_loss(gamma, nu, alpha, beta, targets, weights=(0.1, 0.01, 0.05, 0.05), eps=1e-8, task_weights=None,
+                   target_mask=None):
+    """losses [5D+2]; with `target_mask` [B,D] (see nig_loss_raw) the pair (losses, N_d [D])."""
+    return _MultiTaskLoss.apply(gamma, nu, alpha, beta, targets, weights, eps, task_weights, target_mask)
 
 
 class _FusedHeadLoss(torch.autograd.Function):
     """evidence [B,D,4] + targets -> (nig_out [7,B,D] (non-differentiable), losses [5D+2]); head and loss fused."""
 
     @staticmethod
-    def forward(ctx, evidence, targets, weights, eps, task_weights):
+    def forward(ctx, evidence, targets, weights, eps, task_weights, target_mask=None):
+        counts = _mask_counts(target_mask, targets)
         losses, grad, nig_out, _ = nig_loss_raw(evidence, None, targets, weights=weights, eps=eps,
-                                                task_weights=task_weights, want_nig=True)
+                                                task_weights=task_weights, want_nig=True, target_mask=target_mask,
+                                                counts=counts)
         ctx.save_for_backward(grad)
         ctx.mark_non_differentiable(nig_out)
-        return nig_out, losses
+        if counts is None:
+            return nig_out, losses
+        ctx.mark_non_differentiable(counts)
+        return nig_out, losses, counts
 
     @staticmethod
-    def backward(ctx, _dnig, dlosses):
+    def backward(ctx, _dnig, dlosses, *_dcounts):
         (grad,) = ctx.saved_tensors
         D = grad.shape[1]
-        return grad * dlosses[5 * D + 1], None, None, None, None
+        return grad * dlosses[5 * D + 1], None, None, None, None, None
 
 
-def fused_head_loss(evidence, targets, weights=(0.1, 0.01, 0.05, 0.05), eps=1e-8, task_weights=None):
-    return _FusedHeadLoss.apply(evidence, targets, weights, eps, task_weights)
+def fused_head_loss(evidence, targets, weights=(0.1, 0.01, 0.05, 0.05), eps=1e-8, task_weights=None,
+                    target_mask=None):
+    """(nig_out, losses); with `target_mask` [B,D] (see nig_loss_raw) (nig_out, losses, N_d [D]).  nig_out covers
+    every entry, labelled or not."""
+    return _FusedHeadLoss.apply(evidence, targets, weights, eps, task_weights, target_mask)
 
 
 class _AminiLoss(torch.autograd.Function):

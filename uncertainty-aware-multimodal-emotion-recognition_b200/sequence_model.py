@@ -120,8 +120,12 @@ class SequenceDEERModel(nn.Module):
             st[(dev, name)] = torch.cuda.Stream(device=dev, priority=priority)
         return st[(dev, name)]
 
-    def compute_loss(self, predictions: Dict[str, torch.Tensor], targets: torch.Tensor) -> Dict[str, torch.Tensor]:
-        return self.loss_fn(predictions, targets)
+    def compute_loss(self, predictions: Dict[str, torch.Tensor], targets: torch.Tensor,
+                     target_mask: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
+        """`target_mask` (targets' shape, bool / uint8, nonzero = labelled): partially labelled batch, see losses."""
+        if target_mask is None:
+            return self.loss_fn(predictions, targets)
+        return self.loss_fn(predictions, targets, target_mask=target_mask)
 
     @staticmethod
     def get_predictions_and_uncertainties(outputs: Dict[str, torch.Tensor]):

@@ -8,7 +8,10 @@ groups, :176-245 train_epoch, :219 clip_grad_norm_, :224 optimizer.step).  The r
     clip+AdamW launches (one per LR group) with the clip coefficient computed on the device - no host syncs;
   * the DEER loss is evaluated with exact GLOBAL-batch semantics: its 3x40 sufficient statistics (ECE bins, batch
     means) are all-reduced between the two loss phases, so N ranks x B/N samples give the same loss and gradients as
-    one rank with B samples (BatchNorm statistics in the video encoder stay per-replica, as in stock DDP).
+    one rank with B samples (BatchNorm statistics in the video encoder stay per-replica, as in stock DDP);
+  * partially labelled batches: the optional batch key "target_mask" (targets' shape, bool / uint8, nonzero =
+    labelled) reaches the fused loss; the per-dimension label counts are part of those statistics, so they are global
+    too, and the mask is read on the device only (a captured step picks up a new mask content on every replay).
 """
 from __future__ import annotations
 
@@ -236,6 +239,7 @@ class DEERDataParallelTrainer:
         out = model(batch)   # both models accept the reference's batch dict (preprocessing.py:461-491)
         ev = out[EVIDENCE_KEY]
         targets = batch["targets"]
+        target_mask = batch.get("target_mask")
         B = targets.shape[0]
         hook = self._allreduce if (self.exact_global_loss and self.world > 1) else None
         gb = B * self.world if self.exact_global_loss else B
@@ -244,7 +248,8 @@ class DEERDataParallelTrainer:
         ops.mark("head_out")
         losses, dE, _, _ = ops.nig_loss_raw(ev.detach(), None, targets, weights=self.loss_weights, eps=self.loss_eps,
                                             task_weights=self.task_weights, want_grad=True,
-                                            grad_scale=scale, stats_hook=hook, global_batch=gb)
+                                            grad_scale=scale, stats_hook=hook, global_batch=gb,
+                                            target_mask=target_mask)
         ops.mark("loss_done")
         works = []
         handles = []
